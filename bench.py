@@ -5,6 +5,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...      # the CPU baseline arm (oracle port; TF is not installable)
+    python bench.py ... --dump-outputs DIR    # also write the last timed step's outputs as DIR/<name>.npy
 
 A "step" = one full optimiser step (forward + loss + backward + DP exchange + Adam) of xDeepFM
 (`linear + cin_nets + dnn_nets`, CIN 128x128x128) on one batch of 65 536 rows per GPU: 13 dense +
@@ -61,7 +62,7 @@ CIN_BYTES_PER_ROW = 4 * F_FIELDS + 4 * F_FIELDS * EMB_DIM + 4 * (64 + 64 + 128) 
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
-    ap.add_argument('--steps', type=int, default=20)
+    ap.add_argument('--steps', type=int, default=20, help='timed steps of every timed loop (at least 1)')
     ap.add_argument('--warmup', type=int, default=5)
     ap.add_argument('--impl', default='b200', choices=['b200', 'reference'])
     ap.add_argument('--config', default='xdeepfm', choices=sorted(CONFIGS),
@@ -76,7 +77,15 @@ def parse_args():
                     help='profiling only: experiment build of the CIN backward kernels (cin_tc.cu), 0 = product kernels')
     ap.add_argument('--id-dist', default='uniform', choices=['uniform', 'zipf'],
                     help="categorical id distribution of the synthetic batches (the headline is 'uniform')")
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write what the last timed train step computed to DIR/<name>.npy (rank 0), so that two builds '
+                         'can be compared output for output on the same seeded inputs (b200 arm only)')
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs writes the outputs of the b200 arm; --impl reference has none to write')
+    return args
 
 
 def config_overrides(name, cin_precision=0):
@@ -203,11 +212,12 @@ def measured_peaks():
     return {'hbm_gbs': 6650.0, 'bf16_tflops': 1590.0, 'bf16_tflops_sustained': 1400.0, 'source': 'fallback'}
 
 
-def cpu_baseline(args, conf, steps=None):
+def cpu_baseline(args, conf, steps, warmup=1):
     """The reference's CPU path: TF/Keras cannot be installed here, so this is the oracle PORT (torch CPU fp32
     restatement of the identical graph) on the host cores, on a bounded sample of the same workload: one micro-batch
     of `--cpu-sample-rows` rows of the config's batch (the reference formulation materialises 7 GB per CIN layer at
-    65 536 rows), table rows capped at 100 k per field (per-row work does not depend on the table size)."""
+    65 536 rows), table rows capped at 100 k per field (per-row work does not depend on the table size).
+    Exactly `steps` train steps are timed, after `warmup` (at least one) untimed ones."""
     import torch
     from oracle import model_ref as M
     spec = CONFIGS[args.config]
@@ -231,17 +241,15 @@ def cpu_baseline(args, conf, steps=None):
         cal[nt] = time.perf_counter() - t0
     threads = min(cal, key=cal.get)
     torch.set_num_threads(threads)
-    t0 = time.perf_counter()
-    tr.train_step(idx, dense, y[:, 0])                    # warm-up step, also sizes the sample
-    first = time.perf_counter() - t0
-    budget = 25.0                                         # seconds of CPU work for the timed sample
-    n = max(1, min(steps or 3, int(budget / max(first, 1e-3))))
-    t0 = time.perf_counter()
-    for _ in range(n):
+    warmup = max(1, warmup)
+    for _ in range(warmup):
         tr.train_step(idx, dense, y[:, 0])
-    dt = (time.perf_counter() - t0) / n
-    return {'value': rows / dt, 'unit': 'rows/s', 'cores': threads, 'kind': 'port',
-            'sample': f'{n} train steps x {rows} rows (one micro-batch of the {spec["batch"]}-row batch), {threads} threads = '
+    t0 = time.perf_counter()
+    for _ in range(steps):
+        tr.train_step(idx, dense, y[:, 0])
+    dt = (time.perf_counter() - t0) / steps
+    return {'value': rows / dt, 'unit': 'rows/s', 'cores': threads, 'kind': 'port', 'steps': steps, 'warmup': warmup,
+            'sample': f'{steps} train steps x {rows} rows (one micro-batch of the {spec["batch"]}-row batch), {threads} threads = '
                       f'fastest of a calibration over {sorted(cal)} on {cores} host cores (all {cores} cores: '
                       f'{cal[max(cal)] / cal[threads]:.2f}x slower on the calibration slice), {args.config}, vocab '
                       f'{vocab}/field, torch-CPU fp32 oracle port (TensorFlow not installable: no network)',
@@ -254,14 +262,14 @@ def run_reference(args):
         return
     spec = CONFIGS[args.config]
     conf = reference_config(args.config)              # plain dict: nothing of the product package is imported
-    base = cpu_baseline(args, conf, steps=max(1, args.steps))
+    base = cpu_baseline(args, conf, args.steps, args.warmup)
     assert 'deeptables_b200' not in sys.modules, 'the reference arm must not load the product library'
     line = {'impl': 'reference', 'metric': spec['metric'], 'value': base['value'],
-            'unit': 'rows/s', 'n_gpus': args.gpus, 'steps': args.steps, 'warmup': args.warmup,
+            'unit': 'rows/s', 'n_gpus': args.gpus, 'steps': base['steps'], 'warmup': base['warmup'],
             'ms_per_step': base['sec_per_step'] * 1e3, 'higher_is_better': True, 'scaling': 'weak',
             'vs_baseline': None, 'dtype': 'f32', 'data': 'synthetic',
             'config': {'workload': spec['workload'] + '; CPU sample', 'global_batch': min(args.cpu_sample_rows, spec['batch'])},
-            'cpu_baseline': {k: base[k] for k in ('value', 'unit', 'cores', 'kind', 'sample')},
+            'cpu_baseline': {k: base[k] for k in ('value', 'unit', 'cores', 'kind', 'steps', 'sample')},
             'e2e': {'value': base['value'], 'unit': 'rows/s', 'h2d_bytes_per_step': 0, 'd2h_bytes_per_step': 0}}
     print(json.dumps(line))
 
@@ -387,6 +395,40 @@ def time_cin_kernel(model, cat, peaks):
                                         'cin_tc_dgrad_kernel + 3 x cin_tc_wgrad_kernel'}}
 
 
+DUMP_EMB_SAMPLES = 65536          # (row, field) ids of the last batch whose embedding rows --dump-outputs writes
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(model, prob, cat, out_dir):
+    """Write what one train step hands its caller, right after that step: the batch predictions it returns, the summed
+    loss it accumulates (over every step since the model was built), the dense parameters and buffers after the Adam
+    update, and the embedding rows of a fixed, seeded sample of the batch's ids.  Only rows the step touched are
+    sampled: with lazy Adam the rest of the table is brought up to date only when it is next read.  When the predictions
+    of a large --batch would take the files past DUMP_MAX_BYTES, a fixed, seeded sample of their rows is written, in
+    row order.  Float atomics in the gradient reductions make two runs agree to round-off grown by the training steps,
+    not bit for bit: two runs with the default arguments (5 warm-up + 20 timed xDeepFM steps), compared file by file,
+    gave predictions within 1.2e-3 of each other on one B200 at its 1000 W power limit."""
+    import numpy as np
+    import torch
+    t, scope = model.table, model._scope
+    g = torch.Generator().manual_seed(0)
+    pos = torch.randint(0, cat.numel(), (min(DUMP_EMB_SAMPLES, cat.numel()),), generator=g).to(cat.device)
+    rows = cat.reshape(-1)[pos].long() + t.row_offsets[pos % cat.shape[1]]
+    arrays = {'loss_sum': model._loss_acc.double(), 'dense_params': scope.flat_p,
+              'embedding_rows': t.weight.index_select(0, rows)}
+    if scope.buffers:
+        arrays['dense_buffers'] = torch.cat([b.reshape(-1).float() for b in scope.buffers.values()])
+    room = (DUMP_MAX_BYTES - sum(v.numel() * v.element_size() for v in arrays.values())) // (4 * prob[0].numel())
+    if prob.shape[0] > room:
+        keep = torch.randperm(prob.shape[0], generator=g)[:room].sort().values.to(prob.device)
+        prob = prob.index_select(0, keep)
+    arrays['predictions'] = prob.float()
+    arrays = {k: v.detach().cpu().numpy() for k, v in arrays.items()}
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, f'{k}.npy'), a)
+
+
 def main():
     args = parse_args()
     if args.impl == 'reference':
@@ -442,9 +484,11 @@ def main():
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
         return float(ms.item()) * 1e-3
 
+    last = {}
+
     def dev_step(s):
         c, d, y = devb[s % n_pool]
-        model.train_step(c, d, y)
+        last['prob'] = model.train_step(c, d, y)
 
     def e2e_step(s):
         c, d, y = host[s % n_pool]
@@ -459,6 +503,9 @@ def main():
     secs = timed(dev_step, args.steps)
     launches = N.lib.dtb_launch_count() - l0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        # before the e2e steps below train the model further (and, under a CUDA graph, overwrite the same predictions)
+        dump_outputs(model, last['prob'], devb[(args.steps - 1) % n_pool][0], args.dump_outputs)
     for s in range(2):
         e2e_step(s)
     secs_e2e = timed(e2e_step, args.steps)
@@ -514,8 +561,8 @@ def main():
             'score_only': score,
         }
         if world == 1 and not args.no_cpu_baseline:
-            base = cpu_baseline(args, reference_config(args.config))
-            line['cpu_baseline'] = {k: base[k] for k in ('value', 'unit', 'cores', 'kind', 'sample')}
+            base = cpu_baseline(args, reference_config(args.config), args.steps)
+            line['cpu_baseline'] = {k: base[k] for k in ('value', 'unit', 'cores', 'kind', 'steps', 'sample')}
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()

@@ -119,7 +119,7 @@ def test_bench_reference_arm_prints_the_contract_line():
     import subprocess
     import sys
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    out = subprocess.run([sys.executable, os.path.join(root, 'bench.py'), '--impl', 'reference', '--steps', '1',
+    out = subprocess.run([sys.executable, os.path.join(root, 'bench.py'), '--impl', 'reference', '--steps', '2',
                           '--warmup', '0', '--cpu-sample-rows', '128'], capture_output=True, text=True, timeout=300)
     assert out.returncode == 0, out.stderr[-2000:]
     line = json.loads(out.stdout.strip().splitlines()[-1])
@@ -127,6 +127,11 @@ def test_bench_reference_arm_prints_the_contract_line():
     for key in ('metric', 'n_gpus', 'steps', 'warmup', 'ms_per_step', 'higher_is_better', 'config', 'cpu_baseline', 'e2e'):
         assert key in line, key
     assert line['e2e']['h2d_bytes_per_step'] == 0 and line['cpu_baseline']['kind'] in ('port', 'reference')
+    assert line['steps'] == line['cpu_baseline']['steps'] == 2          # --steps is the number of steps timed
+    assert line['warmup'] == 1                                           # the one untimed step it always runs
+    out = subprocess.run([sys.executable, os.path.join(root, 'bench.py'), '--impl', 'reference', '--dump-outputs', 'x'],
+                         capture_output=True, text=True, timeout=300)
+    assert out.returncode != 0 and '--dump-outputs' in out.stderr
 
 
 def test_ctypes_signatures_match_the_header_prototypes():
