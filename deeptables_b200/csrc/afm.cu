@@ -7,14 +7,13 @@
 //
 // 99 kFLOP per row against 1.7 KB of embedding rows: CUDA-core arithmetic out of shared memory, no tensor-core shape.
 // Forward and the score half of the backward: one WARP per batch row, lanes = pairs (the softmax needs all pairs of a row).
-// Embedding gradient: one THREAD per (row, field) -- it visits the F-1 pairs of its field, recomputes the pair's attention
-// vector, and keeps d e_f in registers (one vector RED per 4 floats at the end; every pair is visited from both ends,
-// which costs 2x the attention FLOPs and saves the scatter).  Attention-kernel gradient: warps stream (row, pair) outer
+// The per-pair backward writes da_p and dv_p = d v_p once per pair.  Embedding gradient: one THREAD per (row, field) -- it
+// sums dv_p * e_other over the F-1 pairs of its field and keeps d e_f in registers (one vector RED per 4 floats at the end;
+// every pair is read from both ends, which saves the scatter).  Attention-kernel gradient: warps stream (row, pair) outer
 // products v_p (x) da_p into register accumulators, lane = (d, group of h).
 // Widths are template parameters: DT = D in {4, 8, 16, 32}; HT = H rounded up to {8, 16, 32} with zero-padded columns
 // (a padded unit has a = act(0) = 0 for relu / linear and h = 0, so it contributes nothing).
 #include "dtb_common.cuh"
-#include <cstdlib>
 
 namespace dtb {
 
@@ -101,9 +100,8 @@ __host__ __device__ inline size_t afm_row_smem_floats(int F, int P, int DT, int 
 }
 
 // MODE 0: pooled[row, :] = sum_p softmax_p v_p.
-// MODE 1: given g = dLoss/d pooled[row, :], writes w_p and ds_p = w_p (g.v_p - sum_q w_q g.v_q) to w_out / ds_out [B, P]
-//         (first backward: afm_bwd_de_kernel then recomputes the attention vector of every pair from both of its fields).
-// MODE 2: the whole per-pair backward, each pair once: da_p[h] = ds_p h[h] act'(a_p[h]) -> w_out [B, P, HT],
+// MODE 2: given g = dLoss/d pooled[row, :], the whole per-pair backward, each pair once: ds_p = w_p (g.v_p - sum_q w_q g.v_q),
+//         da_p[h] = ds_p h[h] act'(a_p[h]) -> w_out [B, P, HT],
 //         dv_p[d] = g[d] w_p + sum_h da_p[h] Wa[d][h] -> ds_out [B, P, DT], d h += ds_p a_p (afm_bwd_gather_kernel finishes).
 template <int DT, int HT, int MODE>
 __global__ void __launch_bounds__(kAfmWarps * 32) afm_rows_kernel(const int32_t* __restrict__ idx, const float* __restrict__ table,
@@ -194,14 +192,7 @@ __global__ void __launch_bounds__(kAfmWarps * 32) afm_rows_kernel(const int32_t*
     }
     sum = warp_sum(sum);
     const float inv = 1.f / sum;
-    if (MODE == 1) {
-      const float delta = warp_sum(dsum) * inv;
-      for (int p = lane; p < P; p += 32) {
-        const float w = sc[p] * inv;
-        w_out[(size_t)row * P + p] = w;
-        ds_out[(size_t)row * P + p] = w * (dw[p] - delta);
-      }
-    } else if (MODE == 2) {
+    if (MODE == 2) {
       const float delta = warp_sum(dsum) * inv;
       for (int p = lane; p < P; p += 32) {
         const float w = sc[p] * inv;
@@ -300,106 +291,6 @@ __global__ void __launch_bounds__(kAfmRows) afm_bwd_gather_kernel(const int32_t*
     }
   }
 }
-
-#ifdef DTB_FIRST_VERSIONS
-// (first backward, compiled only with -DDTB_FIRST_VERSIONS: tools/build_experiments.sh)
-// thread = (row, field f); grid (F, row-chunk groups).  For each other field o: pair p, v = e_f * e_o, a = act(v Wa + ba),
-// da[h] = ds_p h[h] act'(a[h]), dv[d] = g[d] w_p + sum_h da[h] Wa[d][h], d e_f += dv * e_o.
-// The f < o visit also writes da to da_out [B, P, HT] (read by the attention-kernel gradient) and adds ds_p a to d h.
-template <int DT, int HT>
-__global__ void __launch_bounds__(kAfmRows, 2) afm_bwd_de_kernel(const int32_t* __restrict__ idx, const float* __restrict__ table,
-                                                              const int64_t* __restrict__ row_offsets,
-                                                              const float* __restrict__ wa, const float* __restrict__ ba,
-                                                              const float* __restrict__ hv, const float* __restrict__ g,
-                                                              const float* __restrict__ w_in, const float* __restrict__ ds_in,
-                                                              float* __restrict__ da_out, float* __restrict__ grad_table,
-                                                              float* __restrict__ d_hv, int B, int F, int P, int H, int act) {
-  __shared__ __align__(16) float s_wa[DT * HT];
-  __shared__ __align__(16) float s_ba[HT];
-  __shared__ __align__(16) float s_hv[HT];
-  __shared__ float s_dh[HT];
-  afm_stage_weights<DT, HT>(wa, ba, hv, H, s_wa, s_ba, s_hv);
-  for (int h = threadIdx.x; h < HT; h += blockDim.x) s_dh[h] = 0.f;
-  __syncthreads();
-  const int f = blockIdx.x;
-  float dh_acc[HT];
-#pragma unroll
-  for (int h = 0; h < HT; ++h) dh_acc[h] = 0.f;
-  const int n_chunks = (B + kAfmRows - 1) / kAfmRows;
-  for (int chunk = blockIdx.y; chunk < n_chunks; chunk += gridDim.y) {
-    const int row = chunk * kAfmRows + threadIdx.x;
-    if (row >= B) continue;
-    const int64_t rb = table_row(row_offsets, f, __ldg(idx + (int64_t)row * F + f), DT, nullptr);
-    float ef[DT], gr[DT], acc[DT], eo[DT];       // an out-of-range id reads as a zero row and receives no gradient
-#pragma unroll
-    for (int c = 0; c < DT / 4; ++c) {
-      const float4 t = rb >= 0 ? __ldg(reinterpret_cast<const float4*>(table + rb) + c) : make_float4(0.f, 0.f, 0.f, 0.f);
-      ef[4 * c] = t.x; ef[4 * c + 1] = t.y; ef[4 * c + 2] = t.z; ef[4 * c + 3] = t.w;
-      const float4 u = __ldg(reinterpret_cast<const float4*>(g + (size_t)row * DT) + c);
-      gr[4 * c] = u.x; gr[4 * c + 1] = u.y; gr[4 * c + 2] = u.z; gr[4 * c + 3] = u.w;
-      acc[4 * c] = acc[4 * c + 1] = acc[4 * c + 2] = acc[4 * c + 3] = 0.f;
-    }
-    for (int q = 0; q < F - 1; ++q) {
-      const int o = q < f ? q : q + 1;
-      const int p = o < f ? afm_pair_index(o, f, F) : afm_pair_index(f, o, F);
-      const int64_t ro = table_row(row_offsets, o, __ldg(idx + (int64_t)row * F + o), DT, nullptr);
-      const float wp = __ldg(w_in + (size_t)row * P + p), ds = __ldg(ds_in + (size_t)row * P + p);
-      if (ro >= 0) {
-#pragma unroll
-        for (int c = 0; c < DT / 4; ++c) {
-          const float4 t = __ldg(reinterpret_cast<const float4*>(table + ro) + c);
-          eo[4 * c] = t.x; eo[4 * c + 1] = t.y; eo[4 * c + 2] = t.z; eo[4 * c + 3] = t.w;
-        }
-      } else {
-#pragma unroll
-        for (int d = 0; d < DT; ++d) eo[d] = 0.f;
-      }
-      float a[HT];
-      afm_score<DT, HT>(ef, eo, s_wa, s_ba, s_hv, act, a);
-      float hvr[HT];
-      afm_lds<HT>(s_hv, hvr);
-#pragma unroll
-      for (int h = 0; h < HT; ++h) {
-        if (f < o) dh_acc[h] = fmaf(ds, a[h], dh_acc[h]);
-        const float slope = (act == DTB_ACT_RELU && !(a[h] > 0.f)) ? 0.f : 1.f;
-        a[h] = ds * hvr[h] * slope;              // a[] now holds da
-      }
-      if (f < o) {
-        float4* dst = reinterpret_cast<float4*>(da_out + ((size_t)row * P + p) * HT);
-#pragma unroll
-        for (int c = 0; c < HT / 4; ++c) dst[c] = make_float4(a[4 * c], a[4 * c + 1], a[4 * c + 2], a[4 * c + 3]);
-      }
-#pragma unroll
-      for (int d = 0; d < DT; ++d) {
-        float w[HT];
-        afm_lds<HT>(s_wa + d * HT, w);
-        float dv = gr[d] * wp;
-#pragma unroll
-        for (int h = 0; h < HT; ++h) dv = fmaf(a[h], w[h], dv);
-        acc[d] = fmaf(dv, eo[d], acc[d]);
-      }
-    }
-    if (rb >= 0) {
-      float4* dst = reinterpret_cast<float4*>(grad_table + rb);
-#pragma unroll
-      for (int c = 0; c < DT / 4; ++c) {
-        const float4 v = make_float4(acc[4 * c], acc[4 * c + 1], acc[4 * c + 2], acc[4 * c + 3]);
-        if (v.x != 0.f || v.y != 0.f || v.z != 0.f || v.w != 0.f) atomicAdd(dst + c, v);
-      }
-    }
-  }
-  // d projection_h: warp sums -> shared -> one atomic per unit per CTA
-#pragma unroll
-  for (int h = 0; h < HT; ++h) {
-    const float t = warp_sum(dh_acc[h]);
-    if ((threadIdx.x & 31) == 0 && t != 0.f) atomicAdd(&s_dh[h], t);
-  }
-  __syncthreads();
-  for (int h = threadIdx.x; h < H; h += blockDim.x)
-    if (s_dh[h] != 0.f) atomicAdd(d_hv + h, s_dh[h]);
-}
-
-#endif  // DTB_FIRST_VERSIONS
 
 // d Wa[d][h] = sum_{row, p} v_p[d] da_p[h],  d ba[h] = sum da_p[h].  One warp streams rows; lane = (d, group of G = DT*HT/32 units).
 template <int DT, int HT>
@@ -502,7 +393,7 @@ extern "C" {
 size_t dtb_afm_workspace_bytes(int B, int F, int D, int H) {
   if (B <= 0 || F < 2 || H < 1 || H > 32 || D < 1) return 0;
   const size_t P = (size_t)F * (F - 1) / 2;
-  const size_t per_pair = afm_ht(H) + (size_t)(D > 2 ? D : 2);      // da + dv per pair (or da + w + ds on the first path)
+  const size_t per_pair = afm_ht(H) + (size_t)D;      // da + dv per pair
   return (size_t)B * P * per_pair * sizeof(float) + 256;
 }
 
@@ -556,11 +447,6 @@ int dtb_afm_bwd(const int32_t* idx, const float* table, const int64_t* row_offse
                 "workspace missing, misaligned or smaller than dtb_afm_workspace_bytes");
   const int P = F * (F - 1) / 2, HT = afm_ht(H);
   cudaStream_t st = (cudaStream_t)stream;
-  float* w_s = reinterpret_cast<float*>(workspace);
-  float* ds_s = w_s + (size_t)B * P;
-  float* da_s = ds_s + (size_t)B * P;
-  // the da block must start 16-byte aligned: 2 * B * P floats is a multiple of 4 only when B * P is even
-  if ((2 * (size_t)B * P) % 4) da_s += 4 - (2 * (size_t)B * P) % 4;
   int nw = kAfmWarps, nw_w = kAfmWarps;
   while (nw > 1 && afm_row_smem_floats(F, P, D, HT, nw) * sizeof(float) > kAfmSmemMax) nw /= 2;
   auto dw_smem = [&](int n) { return ((size_t)afm_p4(P) + (size_t)n * ((size_t)F * (D + 4) + 32 * HT)) * sizeof(float); };
@@ -573,45 +459,21 @@ int dtb_afm_bwd(const int32_t* idx, const float* table, const int64_t* row_offse
   }
   int grid = sm_count() * 4;
   if (grid > ceil_div(B, nw)) grid = ceil_div(B, nw);
-  int groups = ceil_div(sm_count() * 6, F);
-  if (groups > ceil_div(B, kAfmRows)) groups = ceil_div(B, kAfmRows);
-  // DTB_AFM_BWD=1 selects the first backward (every pair recomputed from both of its fields in afm_bwd_de_kernel; only in
-  // builds with -DDTB_FIRST_VERSIONS)
-  static const int mode = [] { const char* e = getenv("DTB_AFM_BWD"); return e ? atoi(e) : 2; }();
-#ifndef DTB_FIRST_VERSIONS
-  if (mode == 1) {
-    set_error("dtb_afm_bwd: DTB_AFM_BWD=1 needs a library built with -DDTB_FIRST_VERSIONS");
-    return DTB_ERR_UNSUPPORTED;
-  }
-#endif
-  float* da2 = reinterpret_cast<float*>(workspace);             // MODE 2 layout: da [B, P, HT] | dv [B, P, D]
-  float* dv2 = da2 + (size_t)B * P * HT;
+  int g2 = ceil_div(sm_count() * 8, F);
+  if (g2 > ceil_div(B, kAfmRows)) g2 = ceil_div(B, kAfmRows);
+  int grid_w = sm_count() * 2;
+  if (grid_w > ceil_div(B, nw_w)) grid_w = ceil_div(B, nw_w);
+  float* da = reinterpret_cast<float*>(workspace);              // da [B, P, HT] | dv [B, P, D]
+  float* dv = da + (size_t)B * P * HT;
   DTB_AFM_DISPATCH(D, HT, {
-    if (mode == 1) {
-#ifdef DTB_FIRST_VERSIONS
-      auto k1 = afm_rows_kernel<DT_, HT_, 1>;
-      DTB_CUDA_OK(cudaFuncSetAttribute(k1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      k1<<<grid, nw * 32, smem, st>>>(idx, table, row_offsets, att_kernel, att_bias, projection_h, d_pooled, nullptr, w_s,
-                                             ds_s, nullptr, B, F, P, H, act, nullptr);
-      afm_bwd_de_kernel<DT_, HT_><<<dim3(F, groups), kAfmRows, 0, st>>>(idx, table, row_offsets, att_kernel, att_bias,
-                                                                        projection_h, d_pooled, w_s, ds_s, da_s, grad_table,
-                                                                        d_projection_h, B, F, P, H, act);
-#endif
-    } else {
-      auto k1 = afm_rows_kernel<DT_, HT_, 2>;
-      DTB_CUDA_OK(cudaFuncSetAttribute(k1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      k1<<<grid, nw * 32, smem, st>>>(idx, table, row_offsets, att_kernel, att_bias, projection_h, d_pooled, nullptr, da2,
-                                             dv2, d_projection_h, B, F, P, H, act, nullptr);
-      int g2 = ceil_div(sm_count() * 8, F);
-      if (g2 > ceil_div(B, kAfmRows)) g2 = ceil_div(B, kAfmRows);
-      afm_bwd_gather_kernel<DT_><<<dim3(F, g2), kAfmRows, 0, st>>>(idx, table, row_offsets, dv2, grad_table, B, F, P);
-    }
+    auto k1 = afm_rows_kernel<DT_, HT_, 2>;
+    DTB_CUDA_OK(cudaFuncSetAttribute(k1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    k1<<<grid, nw * 32, smem, st>>>(idx, table, row_offsets, att_kernel, att_bias, projection_h, d_pooled, nullptr, da, dv,
+                                    d_projection_h, B, F, P, H, act, nullptr);
+    afm_bwd_gather_kernel<DT_><<<dim3(F, g2), kAfmRows, 0, st>>>(idx, table, row_offsets, dv, grad_table, B, F, P);
     auto k3 = afm_bwd_dw_kernel<DT_, HT_>;
     DTB_CUDA_OK(cudaFuncSetAttribute(k3, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_w));
-    int grid_w = sm_count() * 2;
-    if (grid_w > ceil_div(B, nw_w)) grid_w = ceil_div(B, nw_w);
-    k3<<<grid_w, nw_w * 32, smem_w, st>>>(idx, table, row_offsets, mode == 1 ? da_s : da2, d_att_kernel, d_att_bias, B, F,
-                                               P, H);
+    k3<<<grid_w, nw_w * 32, smem_w, st>>>(idx, table, row_offsets, da, d_att_kernel, d_att_bias, B, F, P, H);
   })
   DTB_LAUNCH_OK();
   return DTB_OK;

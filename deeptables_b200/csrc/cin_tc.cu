@@ -7,9 +7,9 @@
 // m = p = (row r, dim d), keeps h_k[b, :, d] in REGISTERS across the whole layer (it is that thread's
 // own slice of the previous accumulator), and per K-chunk (one x0 field i, all j) multiplies by the
 // scalar x0[b,i,d], splits the fp32 products into bf16 hi + lo and hands them to the tensor core
-// either through TMEM (tcgen05.st, A-from-TMEM MMA) or through shared memory (canonical no-swizzle
-// K-major core matrices).  W_k is pre-split into bf16 hi/lo and pre-tiled in the UMMA canonical
-// layout by a tiny pack kernel, so a whole K-chunk (<= 32 KB) arrives with ONE bulk async copy.
+// through TMEM (tcgen05.st, A-from-TMEM MMA).  W_k is pre-split into bf16 hi/lo and pre-tiled in the
+// UMMA canonical layout by a tiny pack kernel, so a whole K-chunk (<= 32 KB) arrives with ONE bulk
+// async copy.
 //
 // Precision.  bf16x3: Z_hi*W_hi + Z_lo*W_hi + Z_hi*W_lo, fp32 accumulate in TMEM: relative error
 // ~2^-16 per product -- inside the 1e-3 parity bar with margin (single-pass bf16 is ~4e-3).
@@ -60,7 +60,7 @@ __global__ void cin_tc_pack_kernel(const float* __restrict__ w, uint8_t* __restr
 // A operand of a granule in TMEM: 16 columns hi + 16 columns lo per tile; kStagesA granules x 2 tiles
 // in flight = 256 columns, next to the two 128-column accumulators.  The weight chunk of field i (all
 // Hp hidden fields, hi+lo, <= 32 KB) is one bulk copy and serves both tiles and both granules.
-// ---- fp16 variant: max|W_k| (bit pattern, atomicMax on the int view of non-negative floats) and the scaled pack
+// ---- single-pass fp16 kernels (cin_tc2.cu): max|W_k| (bit pattern, atomicMax on the int view of non-negative floats) and the scaled pack
 __global__ void cin_tc_wmax_kernel(const float* __restrict__ w, int64_t n, int* __restrict__ out) {
   float m = 0.f;
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
@@ -105,12 +105,7 @@ __host__ __device__ inline TcSmemLayout tc_layout(int b_stage_bytes, int F) {
   return l;
 }
 
-// kF16 = true is the single-pass fp16 variant (DTB_CIN_TC_F16X1, not the default): operands in fp16 (11-bit
-// significand; one tensor pass instead of the three of the bf16 split) with exact power-of-two scaling into the fp16
-// range -- per GEMM row for the on-the-fly operand Z (bound max|x0 row| * max|h row|), per layer for the weights --
-// undone on the fp32 accumulator.  tools/cin_precision_study.py: max error 2-6e-4 of the output scale, inside the 1e-3
-// parity bar (bf16 single pass: 1.4-4e-3, outside).  With kF16 = false every `if constexpr` below compiles away.
-template <int D, bool kF16 = false>
+template <int D>
 __global__ void __launch_bounds__(kTcThreads, 1) cin_tc_fwd_kernel(const __grid_constant__ CinTcParams p) {
   constexpr int R = 128 / D;                 // batch rows per M=128 tile
   extern __shared__ __align__(1024) uint8_t smem[];
@@ -177,11 +172,6 @@ __global__ void __launch_bounds__(kTcThreads, 1) cin_tc_fwd_kernel(const __grid_
       // ---- h_0 = x0 (zero padded to Hp[0]) ; training: save x0t ------------------------------
 #pragma unroll
       for (int j = 0; j < kMaxHp; ++j) h[j] = (j < F) ? x0g[((size_t)r * F + j) * D + d] : 0.f;
-      [[maybe_unused]] float xmax = 0.f;           // kF16: max|x0[m, :]| of this GEMM row
-      if constexpr (kF16) {
-#pragma unroll
-        for (int j = 0; j < kMaxHp; ++j) xmax = fmaxf(xmax, fabsf(h[j]));
-      }
       if (p.saved) {
         if (b < p.B && !p.compact) {
           float* dst = p.saved + ((size_t)b * D + d) * F;
@@ -195,18 +185,8 @@ __global__ void __launch_bounds__(kTcThreads, 1) cin_tc_fwd_kernel(const __grid_
       }
       for (int k = 0; k < p.n_layers; ++k) {
         const int Hp = p.Hp[k], L = p.L[k];
-        [[maybe_unused]] float srow = 1.f, inv_acc = 1.f;      // kF16: operand scale of this row, and 1/(srow * s_W)
-        if constexpr (kF16) {
-          float hmax = 0.f;
-#pragma unroll
-          for (int j = 0; j < kMaxHp; ++j) hmax = fmaxf(hmax, fabsf(h[j]));
-          float inv_row, sw, inv_w;
-          tc::pow2_scale_to_1024(xmax * hmax, srow, inv_row);
-          tc::pow2_scale_to_1024(__int_as_float(__ldg(p.wmax + k)), sw, inv_w);
-          inv_acc = inv_row * inv_w;
-        }
         for (int i = 0; i < F; ++i) {
-          const float xi = kF16 ? x0g[((size_t)r * F + i) * D + d] * srow : x0g[((size_t)r * F + i) * D + d];
+          const float xi = x0g[((size_t)r * F + i) * D + d];
 #pragma unroll
           for (int half = 0; half < kMaxHp / kSubK; ++half) {
             if (half * kSubK < Hp) {
@@ -215,29 +195,19 @@ __global__ void __launch_bounds__(kTcThreads, 1) cin_tc_fwd_kernel(const __grid_
               // 32 products of this granule -> packed bf16x2 hi / lo (all computed before the async
               // tcgen05.st are issued, so every store reads registers of its own)
               uint32_t zh[kACols], zl[kACols];
-              if (!(p.dbg & 1)) {
 #pragma unroll
-                for (int q = 0; q < kACols; ++q) {
-                  if constexpr (kF16) {
-                    zh[q] = tc::pack_f16x2(xi * h[half * kSubK + 2 * q], xi * h[half * kSubK + 2 * q + 1]);
-                    zl[q] = 0u;
-                  } else {
-                    tc::split_bf16x2(xi * h[half * kSubK + 2 * q], xi * h[half * kSubK + 2 * q + 1], zh[q], zl[q]);
-                  }
-                }
-              }
+              for (int q = 0; q < kACols; ++q)
+                tc::split_bf16x2(xi * h[half * kSubK + 2 * q], xi * h[half * kSubK + 2 * q + 1], zh[q], zl[q]);
               tc::mbar_wait(&empty_a[sa], pa ^ 1);
               tc::fence_after_thread_sync();
-              if (!(p.dbg & 1)) {
-                const uint32_t a_col = tmem_base + lane_base + 2 * kAccCols + ((sa * 2 + g) * 2) * kACols;
-                tc::tmem_st8v(a_col, zh[0], zh[1], zh[2], zh[3], zh[4], zh[5], zh[6], zh[7]);
-                tc::tmem_st8v(a_col + 8, zh[8], zh[9], zh[10], zh[11], zh[12], zh[13], zh[14], zh[15]);
-                if (p.n_pass > 1) {
-                  tc::tmem_st8v(a_col + kACols, zl[0], zl[1], zl[2], zl[3], zl[4], zl[5], zl[6], zl[7]);
-                  tc::tmem_st8v(a_col + kACols + 8, zl[8], zl[9], zl[10], zl[11], zl[12], zl[13], zl[14], zl[15]);
-                }
-                tc::tmem_wait_st();
+              const uint32_t a_col = tmem_base + lane_base + 2 * kAccCols + ((sa * 2 + g) * 2) * kACols;
+              tc::tmem_st8v(a_col, zh[0], zh[1], zh[2], zh[3], zh[4], zh[5], zh[6], zh[7]);
+              tc::tmem_st8v(a_col + 8, zh[8], zh[9], zh[10], zh[11], zh[12], zh[13], zh[14], zh[15]);
+              if (p.n_pass > 1) {
+                tc::tmem_st8v(a_col + kACols, zl[0], zl[1], zl[2], zl[3], zl[4], zl[5], zl[6], zl[7]);
+                tc::tmem_st8v(a_col + kACols + 8, zl[8], zl[9], zl[10], zl[11], zl[12], zl[13], zl[14], zl[15]);
               }
+              tc::tmem_wait_st();
               tc::fence_before_thread_sync();
               __syncwarp();
               if (lane == 0) tc::mbar_arrive(&full_a[g * kStagesA + sa]);
@@ -267,7 +237,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) cin_tc_fwd_kernel(const __grid_
         }
 #pragma unroll
         for (int cb = 0; cb < kMaxL / 16; ++cb) {
-          if (cb * 16 < L && !(p.dbg & 4)) {
+          if (cb * 16 < L) {
             uint32_t v[16];
             tc::tmem_ld16(tmem_base + lane_base + g * kAccCols + cb * 16, v);
             tc::tmem_wait_ld();
@@ -275,7 +245,6 @@ __global__ void __launch_bounds__(kTcThreads, 1) cin_tc_fwd_kernel(const __grid_
 #pragma unroll
             for (int j = 0; j < 16; ++j) {
               float val = __uint_as_float(v[j]);
-              if constexpr (kF16) val *= inv_acc;
               if (bias) val += __ldg(bias + cb * 16 + j);
               if (p.act == DTB_ACT_RELU) val = fmaxf(val, 0.f);
               o[j] = val;
@@ -365,12 +334,11 @@ __global__ void __launch_bounds__(kTcThreads, 1) cin_tc_fwd_kernel(const __grid_
     for (int st = blockIdx.x; st < n_super; st += gridDim.x) {
       for (int k = 0; k < p.n_layers; ++k) {
         const int Hp = p.Hp[k], L = p.L[k];
-        const uint32_t idesc = kF16 ? tc::make_idesc_f16(128, (uint32_t)L) : tc::make_idesc_bf16(128, (uint32_t)L);
+        const uint32_t idesc = tc::make_idesc_bf16(128, (uint32_t)L);
         const uint32_t lbo_b = (uint32_t)(L >> 3) * 128;       // K-direction core stride of the W image
         const uint32_t img_b = (uint32_t)L * Hp * 2;           // bytes of one (hi or lo) image
         // static part of the W descriptor: LBO, SBO = 128 B, version 1, no swizzle
         const uint64_t desc_hi = ((uint64_t)((lbo_b >> 4) & 0x3FFF) << 16) | ((uint64_t)(128 >> 4) << 32) | ((uint64_t)1 << 46);
-        const int n_pass = (p.dbg & 2) ? 0 : p.n_pass;
         for (int i = 0; i < F; ++i, ++chunk) {
           const uint32_t sb = chunk % kStagesB, pb = (chunk / kStagesB) & 1;
           tc::mbar_wait(&full_b[sb], pb);
@@ -387,7 +355,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) cin_tc_fwd_kernel(const __grid_
                 const uint32_t a_base = tmem_base + 2 * kAccCols + ((sa * 2 + g) * 2) * kACols;
 #pragma unroll
                 for (int pass = 0; pass < 3; ++pass) {
-                  if (pass < n_pass) {
+                  if (pass < p.n_pass) {
                     // pass 0: A_hi*B_hi ; 1: A_lo*B_hi ; 2: A_hi*B_lo
                     const uint32_t a_addr = a_base + (pass == 1 ? kACols : 0);
                     const uint32_t b_img = b_addr + (pass == 2 ? img_b : 0) + (uint32_t)half * 4 * lbo_b;
@@ -523,11 +491,7 @@ __global__ void __launch_bounds__(160, 1) tc_selftest_kernel(const float* __rest
 // ------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------
-static int g_tc_variant = 1;
-static int g_tc_dbg = 0;
-static int g_tc_bwd_fp32 = 0;   // test hook: run the exact-fp32 backward after the tensor-core forward   // 1: A operand through TMEM (default), 0: through shared memory
-
-static int g_tc_f16_v1 = 0;     // test hook (bit 18 of set_variant): fp16 single pass on the one-thread-per-row kernels
+static int g_tc_bwd_fp32 = 0;   // test hook (bit 16 of set_variant): run the exact-fp32 backward after the tensor-core forward
 static int g_tc_full_save = 0;  // test hook (bit 17 of set_variant): keep the fp32 T_k rows in the saved activations
 
 static bool d_supported(int D) { return D == 4 || D == 8 || D == 16 || D == 32; }
@@ -548,7 +512,7 @@ bool cin_tc_supported(const CinShape& s) {
     if (round_up(s.H[k], kSubK) > kMaxHp) return false;
     if (k > 0 && s.H[k] % 4) return false;
   }
-  // shared-memory budget of the default variant
+  // shared-memory budget of the forward kernel
   int bstage = 0;
   for (int k = 0; k < s.n_layers; ++k) {
     const int bytes = 4 * s.L[k] * round_up(s.H[k], kSubK);
@@ -560,7 +524,7 @@ bool cin_tc_supported(const CinShape& s) {
 // precision "auto": the single-pass fp16 kernels of cin_tc2.cu when forward, data gradient and weight gradient all
 // support the shape (and the compact saved-activation format is in force), else the bf16x3 kernels of this file
 bool cin_tc_f16_auto(const CinShape& s) {
-  if (g_tc_f16_v1 || !cin_tc_supported(s) || !cin_tc_compact(s)) return false;
+  if (!cin_tc_supported(s) || !cin_tc_compact(s)) return false;
   CinTcParams f{};
   CinTcBwdParams b{};
   f.F = b.F = s.F; f.n_layers = b.n_layers = s.n_layers; f.n_pass = 1; f.compact = b.compact = 1;
@@ -577,6 +541,14 @@ static size_t wpack_bytes(const CinShape& s) {
   size_t b = 0;
   for (int k = 0; k < s.n_layers; ++k) b += (size_t)s.F * s.L[k] * round_up(s.H[k], kSubK) * 4;
   return b;
+}
+
+// grid of the weight-pack kernels of layer k: one thread per packed element, at most 8 CTAs per SM
+static int pack_grid(const CinShape& s, int Hp, int k) {
+  const int64_t total = (int64_t)s.F * s.L[k] * Hp;
+  int blocks = (int)((total + 255) / 256);
+  if (blocks > sm_count() * 8) blocks = sm_count() * 8;
+  return blocks;
 }
 
 static size_t m_pad_rows(const CinShape& s, int B) {
@@ -602,9 +574,9 @@ size_t cin_tc_workspace_bytes(const CinShape& s, int B, int training) {
   return need;
 }
 
-template <int D, bool kF16 = false>
+template <int D>
 static int launch_fwd(const CinTcParams& p, int smem_bytes, cudaStream_t st) {
-  auto kern = cin_tc_fwd_kernel<D, kF16>;
+  auto kern = cin_tc_fwd_kernel<D>;
   DTB_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes));
   const int R = 128 / D;
   const int n_super = (p.B + 2 * R - 1) / (2 * R);
@@ -650,43 +622,36 @@ int cin_tc_fwd(const CinShape& s, const int32_t* idx, const float* table, const 
     hoff += bt_blocks * p.hid_n[k] * kWgPad;
     p.bias_off[k] = s.b_off[k];
     const size_t chunk = (size_t)s.L[k] * p.Hp[k] * 4;
-    // pack layer k
-    const int64_t total = (int64_t)s.F * s.L[k] * p.Hp[k];
-    int blocks = (int)((total + 255) / 256);
-    if (blocks > sm_count() * 8) blocks = sm_count() * 8;
-    if (f16) {
-      // per-layer max|W_k| -> power-of-two scale, then one fp16 image per chunk (the max words live behind the images)
-      int* wmax = reinterpret_cast<int*>(reinterpret_cast<uint8_t*>(workspace) + wpack_bytes(s)) + k;
-      DTB_CUDA_OK(cudaMemsetAsync(wmax, 0, sizeof(int), st));
-      const int64_t n_w = (int64_t)s.F * s.H[k] * s.L[k];
-      cin_tc_wmax_kernel<<<(int)((n_w + 255) / 256 < 64 ? (n_w + 255) / 256 : 64), 256, 0, st>>>(weights + s.w_off[k], n_w, wmax);
-      DTB_LAUNCH_OK();
-      cin_tc_pack_f16_kernel<<<blocks, 256, 0, st>>>(weights + s.w_off[k], reinterpret_cast<uint8_t*>(workspace) + woff,
-                                                     s.F, s.H[k], p.Hp[k], s.L[k], wmax);
-    } else {
-      cin_tc_pack_kernel<<<blocks, 256, 0, st>>>(weights + s.w_off[k], reinterpret_cast<uint8_t*>(workspace) + woff,
-                                                 s.F, s.H[k], p.Hp[k], s.L[k]);
-    }
-    DTB_LAUNCH_OK();
     woff += chunk * s.F;
     soff += (size_t)B * s.D * s.L[k];
     if ((int)chunk > bstage) bstage = (int)chunk;
   }
   p.b_stage_bytes = bstage;
-  p.dbg = g_tc_dbg;
   p.compact = cin_tc_compact(s) ? 1 : 0;
-  p.wmax = reinterpret_cast<const int*>(reinterpret_cast<const uint8_t*>(workspace) + wpack_bytes(s));
-  const TcSmemLayout lay = tc_layout(bstage, s.F);
-  if (f16) {
-    // two threads per GEMM row (cin_tc2.cu) where the shape allows; bit 18 of dtb_cin_tc_set_variant forces the
-    // one-thread-per-row kernel for A/B timing
-    if (!g_tc_f16_v1 && cin_tc2_fwd_supported(p, s.D)) return cin_tc2_launch_fwd(p, s.D, st);
-    if (s.D != 16) {
-      set_error("dtb_cin_fwd: fp16 single pass: shape outside cin_tc2 and embedding dim %d != 16", s.D);
-      return DTB_ERR_UNSUPPORTED;
-    }
-    return launch_fwd<16, true>(p, lay.total, st);
+  int* wmax = reinterpret_cast<int*>(reinterpret_cast<uint8_t*>(workspace) + wpack_bytes(s));     // behind the images
+  p.wmax = wmax;
+  // the single fp16 pass runs on the two-threads-per-row kernels of cin_tc2.cu only
+  if (f16 && !cin_tc2_fwd_supported(p, s.D)) {
+    set_error("dtb_cin_fwd: fp16 single pass: shape outside cin_tc2 (F=%d D=%d); use precision 0/2", s.F, s.D);
+    return DTB_ERR_UNSUPPORTED;
   }
+  for (int k = 0; k < s.n_layers; ++k) {
+    uint8_t* img = reinterpret_cast<uint8_t*>(workspace) + p.wpack_off[k];
+    const int blocks = pack_grid(s, p.Hp[k], k);
+    if (f16) {
+      // per-layer max|W_k| -> power-of-two scale, then one fp16 image per chunk
+      DTB_CUDA_OK(cudaMemsetAsync(wmax + k, 0, sizeof(int), st));
+      const int64_t n_w = (int64_t)s.F * s.H[k] * s.L[k];
+      cin_tc_wmax_kernel<<<(int)((n_w + 255) / 256 < 64 ? (n_w + 255) / 256 : 64), 256, 0, st>>>(weights + s.w_off[k], n_w, wmax + k);
+      DTB_LAUNCH_OK();
+      cin_tc_pack_f16_kernel<<<blocks, 256, 0, st>>>(weights + s.w_off[k], img, s.F, s.H[k], p.Hp[k], s.L[k], wmax + k);
+    } else {
+      cin_tc_pack_kernel<<<blocks, 256, 0, st>>>(weights + s.w_off[k], img, s.F, s.H[k], p.Hp[k], s.L[k]);
+    }
+    DTB_LAUNCH_OK();
+  }
+  if (f16) return cin_tc2_launch_fwd(p, s.D, st);
+  const TcSmemLayout lay = tc_layout(bstage, s.F);
 #define DTB_TC_LAUNCH(DD) \
   case DD:                \
     return launch_fwd<DD>(p, lay.total, st);
@@ -709,12 +674,14 @@ using namespace dtb;
 extern "C" {
 
 // test hooks (declared in include/deeptables_b200.h)
-int dtb_cin_tc_set_variant(int a_operand_in_tmem) {
-  g_tc_dbg = (a_operand_in_tmem >> 8) & 0xff;     // profiling switches ride in bits 8..15
-  g_tc_bwd_fp32 = (a_operand_in_tmem >> 16) & 1;  // bit 16: exact-fp32 backward
-  g_tc_full_save = (a_operand_in_tmem >> 17) & 1; // bit 17: full (fp32 T_k) saved activations
-  g_tc_f16_v1 = (a_operand_in_tmem >> 18) & 1;    // bit 18: fp16 single pass without the cin_tc2.cu kernels
-  g_tc_variant = (a_operand_in_tmem & 0xff) ? 1 : 0;
+int dtb_cin_tc_set_variant(int flags) {
+  const unsigned unknown = (unsigned)flags & ~(1u | (1u << 16) | (1u << 17));    // bit 0 is accepted and ignored
+  if (unknown) {
+    set_error("dtb_cin_tc_set_variant: unknown flag bit %d (known: 0, 16, 17)", __builtin_ctz(unknown));
+    return DTB_ERR_INVALID_ARG;
+  }
+  g_tc_bwd_fp32 = (flags >> 16) & 1;  // bit 16: exact-fp32 backward
+  g_tc_full_save = (flags >> 17) & 1; // bit 17: full (fp32 T_k) saved activations
   return DTB_OK;
 }
 
@@ -774,7 +741,7 @@ __global__ void cin_tc_pack_t_kernel(const float* __restrict__ w, uint8_t* __res
   }
 }
 
-// experiment 6: ONE fp16 image per chunk (the "hi" slot) of B[n=j][k=l] = W[(i*H + j), l] * s_W
+// single fp16 pass (cin_tc2.cu): ONE fp16 image per chunk (the "hi" slot) of B[n=j][k=l] = W[(i*H + j), l] * s_W
 __global__ void cin_tc_pack_t_f16_kernel(const float* __restrict__ w, uint8_t* __restrict__ out, int F, int H, int Hp,
                                          int L, const int* __restrict__ wmax) {
   float s, inv;
@@ -793,54 +760,27 @@ __global__ void cin_tc_pack_t_f16_kernel(const float* __restrict__ w, uint8_t* _
 }
 
 struct TcBwdSmemLayout {
-  int b_off, x0_off, dx_off, a_off, bar_off, total;
+  int b_off, x0_off, dx_off, bar_off, total;
 };
-// stages / a_hi_bytes differ from the defaults only in experiment 5 of the dgrad kernel (dC_hi operand in shared memory)
-__host__ __device__ inline TcBwdSmemLayout tc_bwd_layout(int b_stage_bytes, int F, int stages = kStagesB,
-                                                         int a_hi_bytes = 0) {
+__host__ __device__ inline TcBwdSmemLayout tc_bwd_layout(int b_stage_bytes, int F) {
   TcBwdSmemLayout l;
   l.b_off = 0;
-  l.x0_off = stages * b_stage_bytes;
+  l.x0_off = kStagesB * b_stage_bytes;
   l.dx_off = l.x0_off + 2 * 128 * F * 4;
   l.bar_off = l.dx_off + 2 * 128 * F * 4;
-  l.a_off = l.bar_off;
-  if (a_hi_bytes > 0) {
-    l.a_off = (l.bar_off + 127) / 128 * 128;
-    l.bar_off = l.a_off + a_hi_bytes;
-  }
   l.bar_off = (l.bar_off + 15) / 16 * 16;
   l.total = l.bar_off + 256;
   return l;
 }
 
-// kExp selects experiment builds of the SAME kernel (profiling only, D = 16, chosen by the high nibble of the
-// dbg byte of dtb_cin_tc_set_variant; tools/cin_once.py DGRAD_EXP=n).  0 = product code (every `if constexpr`
-// below compiles away: its SASS is unchanged by the presence of the experiments).
-//   1: no accumulator read-out and no FMAs (synchronisation + MMA skeleton)      2: read-out but no FMAs
-//   3: software-pipelined read-out (next tcgen05.ld issued before the FMAs of the current 16 columns)
-//   4: no MMA issue (producer + read-out + FMAs only)
-//   5: a REAL variant (correct gradients): the dC_hi operand lives in shared memory (UMMA K-major no-swizzle tile,
-//      LBO 2048 / SBO 128 as in tc_selftest_kernel<false>) and passes 0 and 2 use the SS form; only dC_lo stays in
-//      TMEM (pass 1, TS form).  Tests whether A-from-TMEM operand reads limit the N = 64 MMAs / collide with the
-//      accumulator read-out.  Costs 64 KB of shared memory, so it runs with 3 weight stages instead of 4.
-//   6: a REAL variant: ONE tensor pass on fp16 operands (the counterpart of cin_tc_fwd_kernel<16, true>): the dC row is
-//      scaled by an exact power of two chosen from its own max (a second sweep over the row computes it), the weights
-//      by the per-layer scale of cin_tc_pack_t_f16_kernel; both are undone on dx / dh.  The bf16 hi/lo dC tiles for
-//      wgrad are written as before.
-//   7: 6 + the dC tiles for wgrad are ONE fp16 image (row m scaled by its own t_m), 1/t_m is stored per row in the
-//      free "lo" slot and max|dC_k| in the statistics words: the input of cin_tc_wgrad_kernel<true>.
-template <int D, int kExp = 0>
+template <int D>
 __global__ void __launch_bounds__(kTcThreads, 1) cin_tc_dgrad_kernel(const __grid_constant__ CinTcBwdParams p) {
   constexpr int R = 128 / D;
   extern __shared__ __align__(1024) uint8_t smem[];
-  constexpr bool kF16A = (kExp == 6 || kExp == 7);                   // single fp16 pass (7: also fp16 dC tiles for wgrad)
-  constexpr int kSB = (kExp == 5) ? 3 : kStagesB;                    // weight stages
-  constexpr int kAHiTile = 128 * kMaxL * 2;                           // bytes of one tile's dC_hi operand (experiment 5)
-  const TcBwdSmemLayout lay = tc_bwd_layout(p.b_stage_bytes, p.F, kSB, kExp == 5 ? 2 * kAHiTile : 0);
+  const TcBwdSmemLayout lay = tc_bwd_layout(p.b_stage_bytes, p.F);
   uint8_t* smem_b = smem + lay.b_off;
   float* x0s = reinterpret_cast<float*>(smem + lay.x0_off);
   float* dxs = reinterpret_cast<float*>(smem + lay.dx_off);
-  [[maybe_unused]] uint8_t* smem_a = smem + lay.a_off;
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem + lay.bar_off);
   uint64_t* a_ready = bars;          // [tile]            2
   uint64_t* full_b = bars + 2;       // [stage]           4
@@ -856,7 +796,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) cin_tc_dgrad_kernel(const __gri
   if (threadIdx.x == 0) {
     tc::mbar_init(&a_ready[0], 4);
     tc::mbar_init(&a_ready[1], 4);
-    for (int s = 0; s < kSB; ++s) {
+    for (int s = 0; s < kStagesB; ++s) {
       tc::mbar_init(&full_b[s], 1);
       tc::mbar_init(&empty_b[s], 1);
     }
@@ -922,41 +862,6 @@ __global__ void __launch_bounds__(kTcThreads, 1) cin_tc_dgrad_kernel(const __gri
         }
         const float* dprow = p.d_pooled + (size_t)b * p.P + p.pcol0[k];
         uint8_t* dcblk = p.dc_tiles + p.dc_off[k] + (m_pad >> 4) * (size_t)(64 * L) + ((t & 15) >> 3) * 128 + (t & 7) * 16;
-        [[maybe_unused]] float trow = 1.f, inv_acc = 1.f;      // kExp 6: scale of this dC row, and 1/(trow * s_W)
-        if constexpr (kF16A) {
-          float dmax = 0.f;
-#pragma unroll
-          for (int cb = 0; cb < kMaxL / 16; ++cb) {
-            if (cb * 16 < L) {
-#pragma unroll
-              for (int j = 0; j < 16; ++j) {
-                const int col = cb * 16 + j;
-                float gsum = 0.f;
-                if (valid && col >= pool_lo && col < pool_lo + pool_n) gsum = __ldg(dprow + (col - pool_lo));
-                if (col < kMaxHp) {
-                  if (col < hid_n) gsum += dh[col];
-                }
-                const bool on = p.compact ? (((mw[cb >> 1] >> ((cb & 1) * 16 + j)) & 1u) != 0u)
-                                          : (valid && Trow[col] > 0.f);
-                if (p.act == DTB_ACT_RELU && !on) gsum = 0.f;
-                dmax = fmaxf(dmax, fabsf(gsum));
-              }
-            }
-          }
-          float inv_t, sw, inv_w;
-          tc::pow2_scale_to_1024(dmax, trow, inv_t);
-          tc::pow2_scale_to_1024(__int_as_float(__ldg(p.wmax + k)), sw, inv_w);
-          inv_acc = inv_t * inv_w;
-          if constexpr (kExp == 7) {
-            // wgrad (fp16 variant) folds 1/t_m into its on-the-fly operand: one float per row in the unused "lo"
-            // slot of the row's 16-row tile block; the layer's max|dC| goes to the statistics words (slot 8 + k)
-            *reinterpret_cast<float*>(p.dc_tiles + p.dc_off[k] + (m_pad >> 4) * (size_t)(64 * L) + 32 * L + (t & 15) * 4) = inv_t;
-            float wm = dmax;
-#pragma unroll
-            for (int off = 16; off >= 1; off >>= 1) wm = fmaxf(wm, __shfl_xor_sync(0xffffffffu, wm, off));
-            if (lane == 0 && wm > 0.f) atomicMax(const_cast<int*>(p.wmax) + 8 + k, __float_as_int(wm));
-          }
-        }
 #pragma unroll
         for (int cb = 0; cb < kMaxL / 16; ++cb) {
           if (cb * 16 < L) {
@@ -983,37 +888,16 @@ __global__ void __launch_bounds__(kTcThreads, 1) cin_tc_dgrad_kernel(const __gri
             uint32_t zh[8], zl[8];
 #pragma unroll
             for (int q = 0; q < 8; ++q) tc::split_bf16x2(dc[2 * q], dc[2 * q + 1], zh[q], zl[q]);
-            if constexpr (kExp == 5) {
-              uint8_t* arow = smem_a + g * kAHiTile + (t >> 3) * 128 + (t & 7) * 16;     // k-group stride 2048 B
-              *reinterpret_cast<uint4*>(arow + (2 * cb) * 2048) = make_uint4(zh[0], zh[1], zh[2], zh[3]);
-              *reinterpret_cast<uint4*>(arow + (2 * cb + 1) * 2048) = make_uint4(zh[4], zh[5], zh[6], zh[7]);
-            } else if constexpr (kF16A) {
-              uint32_t zf[8];
-#pragma unroll
-              for (int q = 0; q < 8; ++q) zf[q] = tc::pack_f16x2(dc[2 * q] * trow, dc[2 * q + 1] * trow);
-              tc::tmem_st8v(t_tile + cb * 8, zf[0], zf[1], zf[2], zf[3], zf[4], zf[5], zf[6], zf[7]);
-            } else {
-              tc::tmem_st8v(t_tile + cb * 8, zh[0], zh[1], zh[2], zh[3], zh[4], zh[5], zh[6], zh[7]);
-            }
-            if constexpr (!kF16A)
-              tc::tmem_st8v(t_tile + 64 + cb * 8, zl[0], zl[1], zl[2], zl[3], zl[4], zl[5], zl[6], zl[7]);
-            if constexpr (kExp == 7) {
-              uint32_t zt[8];
-#pragma unroll
-              for (int q = 0; q < 8; ++q) zt[q] = tc::pack_f16x2(dc[2 * q] * trow, dc[2 * q + 1] * trow);
-              *reinterpret_cast<uint4*>(dcblk + (cb * 2) * 256) = make_uint4(zt[0], zt[1], zt[2], zt[3]);
-              *reinterpret_cast<uint4*>(dcblk + (cb * 2 + 1) * 256) = make_uint4(zt[4], zt[5], zt[6], zt[7]);
-            } else {
+            tc::tmem_st8v(t_tile + cb * 8, zh[0], zh[1], zh[2], zh[3], zh[4], zh[5], zh[6], zh[7]);
+            tc::tmem_st8v(t_tile + 64 + cb * 8, zl[0], zl[1], zl[2], zl[3], zl[4], zl[5], zl[6], zl[7]);
             *reinterpret_cast<uint4*>(dcblk + (cb * 2) * 256) = make_uint4(zh[0], zh[1], zh[2], zh[3]);
             *reinterpret_cast<uint4*>(dcblk + (cb * 2 + 1) * 256) = make_uint4(zh[4], zh[5], zh[6], zh[7]);
             *reinterpret_cast<uint4*>(dcblk + 32 * L + (cb * 2) * 256) = make_uint4(zl[0], zl[1], zl[2], zl[3]);
             *reinterpret_cast<uint4*>(dcblk + 32 * L + (cb * 2 + 1) * 256) = make_uint4(zl[4], zl[5], zl[6], zl[7]);
-            }
             tc::tmem_wait_st();
           }
         }
         tc::fence_before_thread_sync();
-        if constexpr (kExp == 5) tc::fence_proxy_async_smem();     // generic-proxy stores -> visible to the UMMA reads
         __syncwarp();
         if (lane == 0) tc::mbar_arrive(&a_ready[g]);
         // ---- h_k (this row's slice) and a fresh dh accumulator ------------------------------------
@@ -1042,60 +926,27 @@ __global__ void __launch_bounds__(kTcThreads, 1) cin_tc_dgrad_kernel(const __gri
         for (int i = 0; i < F; ++i) {
           const uint32_t buf = acc_cnt & 1, par = (acc_cnt >> 1) & 1;
           ++acc_cnt;
-          const float xi = kF16A ? x0g[((size_t)r * F + i) * D + d] * inv_acc : x0g[((size_t)r * F + i) * D + d];
+          const float xi = x0g[((size_t)r * F + i) * D + d];
           tc::mbar_wait(&acc_full[g * 2 + buf], par);
           tc::fence_after_thread_sync();
           float dx = 0.f;
-          if constexpr (kExp == 3) {
-            uint32_t v0[16], v1[16];
-            const uint32_t acc_addr = t_tile + 128 + buf * 64;
-            tc::tmem_ld16(acc_addr, v0);
-#pragma unroll
-            for (int cb = 0; cb < kMaxHp / 16; ++cb) {
-              if (cb * 16 < Hp) {
-                tc::tmem_wait_ld();
-                const bool more = cb + 1 < kMaxHp / 16 && (cb + 1) * 16 < Hp;
-                if (more) {
-                  if (cb & 1) tc::tmem_ld16(acc_addr + (cb + 1) * 16, v0);
-                  else tc::tmem_ld16(acc_addr + (cb + 1) * 16, v1);
-                }
-#pragma unroll
-                for (int j = 0; j < 16; ++j) {
-                  const float dz = __uint_as_float((cb & 1) ? v1[j] : v0[j]);
-                  dx = fmaf(dz, h[cb * 16 + j], dx);
-                  dh[cb * 16 + j] = fmaf(dz, xi, dh[cb * 16 + j]);
-                }
-              }
-            }
-          } else if constexpr (kExp == 1) {
-            dx = xi;
-          } else {
 #pragma unroll
           for (int cb = 0; cb < kMaxHp / 16; ++cb) {
             if (cb * 16 < Hp) {
               uint32_t v[16];
               tc::tmem_ld16(t_tile + 128 + buf * 64 + cb * 16, v);
               tc::tmem_wait_ld();
-              if constexpr (kExp == 2) {
-                uint32_t x = 0;
-#pragma unroll
-                for (int j = 0; j < 16; ++j) x ^= v[j];
-                dx += __uint_as_float(x & 1u);
-              } else {
 #pragma unroll
               for (int j = 0; j < 16; ++j) {
                 const float dz = __uint_as_float(v[j]);
                 dx = fmaf(dz, h[cb * 16 + j], dx);
                 dh[cb * 16 + j] = fmaf(dz, xi, dh[cb * 16 + j]);
               }
-              }
             }
-          }
           }
           tc::fence_before_thread_sync();
           __syncwarp();
           if (lane == 0) tc::mbar_arrive(&acc_empty[g * 2 + buf]);
-          if constexpr (kF16A) dx *= inv_acc;
           dxg[i * 128 + t] += dx;
         }
         if (k == 0) {
@@ -1120,12 +971,12 @@ __global__ void __launch_bounds__(kTcThreads, 1) cin_tc_dgrad_kernel(const __gri
     for (int st = blockIdx.x; st < n_super; st += gridDim.x) {
       for (int k = p.n_layers - 1; k >= 0; --k, ++layer_cnt) {
         const int Hp = p.Hp[k], L = p.L[k];
-        const uint32_t idesc = kF16A ? tc::make_idesc_f16(128, (uint32_t)Hp) : tc::make_idesc_bf16(128, (uint32_t)Hp);
+        const uint32_t idesc = tc::make_idesc_bf16(128, (uint32_t)Hp);
         const uint32_t lbo_b = (uint32_t)(Hp >> 3) * 128;
         const uint32_t img_b = (uint32_t)L * Hp * 2;
         const uint64_t desc_hi = ((uint64_t)((lbo_b >> 4) & 0x3FFF) << 16) | ((uint64_t)(128 >> 4) << 32) | ((uint64_t)1 << 46);
         for (int i = 0; i < F; ++i, ++chunk) {
-          const uint32_t sb = chunk % kSB, pb = (chunk / kSB) & 1;
+          const uint32_t sb = chunk % kStagesB, pb = (chunk / kStagesB) & 1;
           tc::mbar_wait(&full_b[sb], pb);
           const uint32_t b_addr = smem_b_u32 + sb * (uint32_t)p.b_stage_bytes;
 #pragma unroll
@@ -1141,22 +992,14 @@ __global__ void __launch_bounds__(kTcThreads, 1) cin_tc_dgrad_kernel(const __gri
               const uint32_t d_tmem = a_base + 128 + buf * 64;
 #pragma unroll
               for (int pass = 0; pass < 3; ++pass) {
-                if (pass < (kF16A ? 1 : p.n_pass)) {
+                if (pass < p.n_pass) {
                   const uint32_t a_addr = a_base + (pass == 1 ? 64 : 0);
                   const uint32_t b_img = b_addr + (pass == 2 ? img_b : 0);
 #pragma unroll
                   for (int ks = 0; ks < kMaxL / 16; ++ks) {
                     if (ks * 16 < L) {
                       const uint64_t desc_b = desc_hi | (uint64_t)(((b_img + ks * 2 * lbo_b) >> 4) & 0x3FFF);
-                      if constexpr (kExp == 5) {
-                        if (pass == 1)
-                          tc::mma_ts(d_tmem, a_addr + ks * 8, desc_b, idesc, (uint32_t)((pass | ks) != 0));
-                        else
-                          tc::mma_ss(d_tmem, tc::make_smem_desc(tc::smem_u32(smem_a) + g * kAHiTile + ks * 4096, 2048, 128),
-                                     desc_b, idesc, (uint32_t)((pass | ks) != 0));
-                      } else if constexpr (kExp != 4) {
-                        tc::mma_ts(d_tmem, a_addr + ks * 8, desc_b, idesc, (uint32_t)((pass | ks) != 0));
-                      }
+                      tc::mma_ts(d_tmem, a_addr + ks * 8, desc_b, idesc, (uint32_t)((pass | ks) != 0));
                     }
                   }
                 }
@@ -1175,11 +1018,11 @@ __global__ void __launch_bounds__(kTcThreads, 1) cin_tc_dgrad_kernel(const __gri
       uint32_t chunk = 0;
       for (int st = blockIdx.x; st < n_super; st += gridDim.x) {
         for (int k = p.n_layers - 1; k >= 0; --k) {
-          const uint32_t bytes = (uint32_t)p.L[k] * p.Hp[k] * 2 * ((!kF16A && p.n_pass > 1) ? 2 : 1);
+          const uint32_t bytes = (uint32_t)p.L[k] * p.Hp[k] * 2 * (p.n_pass > 1 ? 2 : 1);
           const uint32_t stride = (uint32_t)p.L[k] * p.Hp[k] * 4;
           const uint8_t* src = p.wpack + p.wpack_off[k];
           for (int i = 0; i < F; ++i, ++chunk) {
-            const uint32_t sb = chunk % kSB, pb = (chunk / kSB) & 1;
+            const uint32_t sb = chunk % kStagesB, pb = (chunk / kStagesB) & 1;
             tc::mbar_wait(&empty_b[sb], pb ^ 1);
             tc::mbar_arrive_expect_tx(&full_b[sb], bytes);
             tc::bulk_g2s(smem_b + (size_t)sb * p.b_stage_bytes, src + (size_t)i * stride, bytes, &full_b[sb]);
@@ -1215,8 +1058,6 @@ struct CinTcWgradParams {
   int F, H, Hp, L, n_pass;
   int n_stage_total;         // ceil(M_pad / 64)
   int stages_per_split;
-  const int* stats;          // fp16 variant: [8 + k] max|dC_k|, [16] max|x0 tiles|, [24 + k] max|h_k tiles| (bit patterns)
-  int layer;
 };
 
 struct WgSmemLayout {
@@ -1235,11 +1076,6 @@ __host__ __device__ inline WgSmemLayout wg_layout(int L, int Hp, int F) {
   return l;
 }
 
-// kF16 = true: ONE fp16 pass (input written by cin_tc_dgrad_kernel<16, 7>).  The reduction runs over the batch rows
-// m, so both operands need scales that do not depend on m inside the MMA: the dC tile row m carries its own t_m, which
-// is cancelled on the other operand, A'[(i,j), m] = x0[m,i] h[m,j] (G / t_m), with ONE per-layer G chosen from the
-// recorded maxima so that |A'| < 1024 (rows whose contribution is negligible may underflow, nothing can overflow).
-template <bool kF16 = false>
 __global__ void __launch_bounds__(kWgThreads, 1) cin_tc_wgrad_kernel(const __grid_constant__ CinTcWgradParams p) {
   extern __shared__ __align__(1024) uint8_t smem[];
   const WgSmemLayout lay = wg_layout(p.L, p.Hp, p.F);
@@ -1289,12 +1125,6 @@ __global__ void __launch_bounds__(kWgThreads, 1) cin_tc_wgrad_kernel(const __gri
     const bool live = (i < F) && (j < H);
     const bool h_is_x = (p.hb == p.xb);
     const uint32_t lane_base = (uint32_t)((warp & 3) * 32) << 16;
-    [[maybe_unused]] float gscale = 1.f, inv_g = 1.f;
-    if constexpr (kF16) {
-      const float xm = __int_as_float(__ldg(p.stats + 16)), hm = __int_as_float(__ldg(p.stats + 24 + p.layer));
-      const float dm = __int_as_float(__ldg(p.stats + 8 + p.layer));
-      tc::pow2_scale_to_1024(xm * hm * dm * (1.0f / 512.0f), gscale, inv_g);     // 1/t_m <= max|dC| / 512
-    }
     for (int s = 0; s < n_st; ++s) {
       const uint32_t sh = s % kWgStages, ph = (s / kWgStages) & 1;
       const uint32_t sa = s % kWgStagesA, pa = (s / kWgStagesA) & 1;
@@ -1305,27 +1135,12 @@ __global__ void __launch_bounds__(kWgThreads, 1) cin_tc_wgrad_kernel(const __gri
       const float4* xrow = reinterpret_cast<const float4*>(xs + (live ? i : 0) * kWgPad);
       const float4* hrow = reinterpret_cast<const float4*>(hs + (live ? j : 0) * kWgPad);
       uint32_t zh[32], zl[32];
-      if constexpr (kF16) {
-        // the stage's dC blocks carry 1/t_m of their 16 rows at the head of the unused "lo" slot
-        tc::mbar_wait(&full_b[sh], ph);
-        const float* tv = reinterpret_cast<const float*>(smem + lay.b_off + sh * lay.b_bytes);
-#pragma unroll
-        for (int q4 = 0; q4 < 16; ++q4) {
-          const float4 xv = xrow[q4], hv = hrow[q4];
-          const float4 cv = *reinterpret_cast<const float4*>(tv + (q4 >> 2) * (16 * L) + 8 * L + (q4 & 3) * 4);
-          const float sc = live ? gscale : 0.f;
-          zh[2 * q4] = tc::pack_f16x2(xv.x * hv.x * (cv.x * sc), xv.y * hv.y * (cv.y * sc));
-          zh[2 * q4 + 1] = tc::pack_f16x2(xv.z * hv.z * (cv.z * sc), xv.w * hv.w * (cv.w * sc));
-          zl[2 * q4] = zl[2 * q4 + 1] = 0u;
-        }
-      } else {
 #pragma unroll
       for (int q4 = 0; q4 < 16; ++q4) {
         const float4 xv = xrow[q4], hv = hrow[q4];
         const float sc = live ? 1.f : 0.f;
         tc::split_bf16x2(xv.x * hv.x * sc, xv.y * hv.y * sc, zh[2 * q4], zl[2 * q4]);
         tc::split_bf16x2(xv.z * hv.z * sc, xv.w * hv.w * sc, zh[2 * q4 + 1], zl[2 * q4 + 1]);
-      }
       }
       __syncwarp();
       if (lane == 0) tc::mbar_arrive(&empty_h[sh]);
@@ -1336,8 +1151,7 @@ __global__ void __launch_bounds__(kWgThreads, 1) cin_tc_wgrad_kernel(const __gri
       for (int ks = 0; ks < 4; ++ks) {
         tc::tmem_st8v(a_col + ks * 16, zh[ks * 8 + 0], zh[ks * 8 + 1], zh[ks * 8 + 2], zh[ks * 8 + 3], zh[ks * 8 + 4],
                       zh[ks * 8 + 5], zh[ks * 8 + 6], zh[ks * 8 + 7]);
-        if constexpr (!kF16)
-          tc::tmem_st8v(a_col + ks * 16 + 8, zl[ks * 8 + 0], zl[ks * 8 + 1], zl[ks * 8 + 2], zl[ks * 8 + 3], zl[ks * 8 + 4],
+        tc::tmem_st8v(a_col + ks * 16 + 8, zl[ks * 8 + 0], zl[ks * 8 + 1], zl[ks * 8 + 2], zl[ks * 8 + 3], zl[ks * 8 + 4],
                         zl[ks * 8 + 5], zl[ks * 8 + 6], zl[ks * 8 + 7]);
       }
       tc::tmem_wait_st();
@@ -1358,7 +1172,7 @@ __global__ void __launch_bounds__(kWgThreads, 1) cin_tc_wgrad_kernel(const __gri
           tc::tmem_wait_ld();
           if (live) {
 #pragma unroll
-            for (int q = 0; q < 16; ++q) atomicAdd(dst + cb * 16 + q, kF16 ? __uint_as_float(v[q]) * inv_g : __uint_as_float(v[q]));
+            for (int q = 0; q < 16; ++q) atomicAdd(dst + cb * 16 + q, __uint_as_float(v[q]));
           }
         }
       }
@@ -1366,7 +1180,7 @@ __global__ void __launch_bounds__(kWgThreads, 1) cin_tc_wgrad_kernel(const __gri
     }
   } else if (warp == 8) {
     const bool leader = elect_one_sync();
-    const uint32_t idesc = kF16 ? (tc::make_idesc_f16(128, (uint32_t)L) | (1u << 16)) : tc::make_idesc_bf16_bmn(128, (uint32_t)L);
+    const uint32_t idesc = tc::make_idesc_bf16_bmn(128, (uint32_t)L);
     // dC tile descriptor (MN-major): LBO = 128 B (k-group), SBO = 256 B (n-group)
     const uint64_t desc_hi = ((uint64_t)(128 >> 4) << 16) | ((uint64_t)(256 >> 4) << 32) | ((uint64_t)1 << 46);
     const uint32_t smem_b_u32 = tc::smem_u32(smem + lay.b_off);
@@ -1386,7 +1200,7 @@ __global__ void __launch_bounds__(kWgThreads, 1) cin_tc_wgrad_kernel(const __gri
           for (int ks = 0; ks < 4; ++ks) {
 #pragma unroll
             for (int pass = 0; pass < 3; ++pass) {
-              if (pass < (kF16 ? 1 : p.n_pass)) {
+              if (pass < p.n_pass) {
                 // pass 0: Z_hi*dC_hi ; 1: Z_lo*dC_hi ; 2: Z_hi*dC_lo
                 const uint32_t a_addr = a_base + ks * 16 + (pass == 1 ? 8 : 0);
                 const uint32_t blk = b_addr + ks * (64 * L) + (pass == 2 ? 32 * L : 0);
@@ -1480,9 +1294,9 @@ size_t cin_tc_bwd_workspace_bytes(const CinShape& s, int B) {
   return bwd_stats_end(s, B) + (size_t)B * kCinMaxLayers * sizeof(float) + 256;
 }
 
-template <int D, int kExp>
-static int launch_dgrad_exp(const CinTcBwdParams& p, int smem_bytes, cudaStream_t st) {
-  auto kern = cin_tc_dgrad_kernel<D, kExp>;
+template <int D>
+static int launch_dgrad(const CinTcBwdParams& p, int smem_bytes, cudaStream_t st) {
+  auto kern = cin_tc_dgrad_kernel<D>;
   DTB_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes));
   const int R = 128 / D;
   const int n_super = (p.B + 2 * R - 1) / (2 * R);
@@ -1491,36 +1305,6 @@ static int launch_dgrad_exp(const CinTcBwdParams& p, int smem_bytes, cudaStream_
   kern<<<grid, kTcThreads, smem_bytes, st>>>(p);
   DTB_LAUNCH_OK();
   return DTB_OK;
-}
-
-template <int D>
-static int launch_dgrad(const CinTcBwdParams& p, int smem_bytes, cudaStream_t st) {
-#ifdef DTB_CIN_EXPERIMENTS
-  // experiment builds of the one-thread-per-row kernel (profiling only, see cin_tc_dgrad_kernel): compiled only with
-  // -DDTB_CIN_EXPERIMENTS (tools/build_experiments.sh); the product library holds kExp = 0 alone
-  if constexpr (D == 16) {
-    switch (g_tc_dbg >> 4) {
-      case 1: return launch_dgrad_exp<16, 1>(p, smem_bytes, st);
-      case 2: return launch_dgrad_exp<16, 2>(p, smem_bytes, st);
-      case 3: return launch_dgrad_exp<16, 3>(p, smem_bytes, st);
-      case 4: return launch_dgrad_exp<16, 4>(p, smem_bytes, st);
-      case 6: return launch_dgrad_exp<16, 6>(p, smem_bytes, st);
-      case 7: return launch_dgrad_exp<16, 7>(p, smem_bytes, st);
-      case 5: {
-        const int need = tc_bwd_layout(p.b_stage_bytes, p.F, 3, 2 * 128 * kMaxL * 2).total;
-        if (need <= 227 * 1024) return launch_dgrad_exp<16, 5>(p, need, st);
-        break;
-      }
-      default: break;
-    }
-  }
-#else
-  if ((g_tc_dbg >> 4) != 0) {
-    set_error("dtb_cin_bwd: experiment build %d requested but this library was built without -DDTB_CIN_EXPERIMENTS", g_tc_dbg >> 4);
-    return DTB_ERR_UNSUPPORTED;
-  }
-#endif
-  return launch_dgrad_exp<D, 0>(p, smem_bytes, st);
 }
 
 static bool cin_tc_bwd_supported(const CinShape& s) {
@@ -1561,17 +1345,9 @@ int cin_tc_bwd(const CinShape& s, const int32_t* idx, const float* table, const 
   dc_bytes(s, B, dc_off);
   size_t woff = 0, soff = (size_t)B * s.D * s.F;
   p.compact = cin_tc_compact(s) ? 1 : 0;
-  // experiment builds 6 / 7 (single fp16 pass; profiling hook only): 64 statistics words at the end of the workspace:
-  // [k] max|W_k|, [8 + k] max|dC_k|, [16] max|x0 tiles|, [24 + k] max|h_k tiles|  (bit patterns of non-negative floats)
-  const int exp_build = g_tc_dbg >> 4;
-  // fp16 single pass (DTB_CIN_TC_F16X1): the two-threads-per-row data-gradient kernel of cin_tc2.cu + fp16 dC tiles for
-  // cin_tc_wgrad_kernel<true>.  Decided below once the layer table is filled (cin_tc2_bwd_supported).
-  bool f16_v2 = false;
-  const bool f16a = !f16 && s.D == 16 && (exp_build == 6 || exp_build == 7);
-  bool f16w = !f16 && s.D == 16 && exp_build == 7 && d_bias == nullptr;
-  int* stats = reinterpret_cast<int*>(ws + bwd_stats_end(s, B) - 256);
-  float* dpmax = reinterpret_cast<float*>(ws + bwd_stats_end(s, B));
-  size_t hoff = cin_fp32_saved_bytes(s, B) / sizeof(float) + (m_pad_rows(s, B) / 64) * s.F * kWgPad;   // as cin_tc_fwd
+  const size_t bt_blocks = m_pad_rows(s, B) / 64;
+  const size_t xb_pos = cin_fp32_saved_bytes(s, B) / sizeof(float);      // block-transposed tiles, as cin_tc_fwd
+  size_t hoff = xb_pos + bt_blocks * s.F * kWgPad;
   int bstage = 0;
   for (int k = 0; k < s.n_layers; ++k) {
     p.L[k] = s.L[k]; p.H[k] = s.H[k]; p.Hp[k] = round_up(s.H[k], kSubK);
@@ -1579,37 +1355,24 @@ int cin_tc_bwd(const CinShape& s, const int32_t* idx, const float* table, const 
     p.hid_n[k] = (k + 1 < s.n_layers) ? s.H[k + 1] : 0;
     p.wpack_off[k] = woff; p.saved_off[k] = soff; p.dc_off[k] = dc_off[k];
     p.hb_off[k] = hoff;
-    hoff += (m_pad_rows(s, B) / 64) * p.hid_n[k] * kWgPad;
+    hoff += bt_blocks * p.hid_n[k] * kWgPad;
     const size_t chunk = (size_t)s.L[k] * p.Hp[k] * 4;
-    const int64_t total = (int64_t)s.F * s.L[k] * p.Hp[k];
-    int blocks = (int)((total + 255) / 256);
-    if (blocks > sm_count() * 8) blocks = sm_count() * 8;
-    if (phase != 2 && !f16) {
-      if (f16a) {                                    // experiments 6 / 7: scaled fp16 weights; statistics words in the trailing slack
-        int* wmax = stats + k;
-        if (k == 0) DTB_CUDA_OK(cudaMemsetAsync(stats, 0, 256, st));
-        const int64_t n_w = (int64_t)s.F * s.H[k] * s.L[k];
-        cin_tc_wmax_kernel<<<(int)((n_w + 255) / 256 < 64 ? (n_w + 255) / 256 : 64), 256, 0, st>>>(weights + s.w_off[k], n_w, wmax);
-        DTB_LAUNCH_OK();
-        cin_tc_pack_t_f16_kernel<<<blocks, 256, 0, st>>>(weights + s.w_off[k], ws + woff, s.F, s.H[k], p.Hp[k], s.L[k], wmax);
-      } else {
-        cin_tc_pack_t_kernel<<<blocks, 256, 0, st>>>(weights + s.w_off[k], ws + woff, s.F, s.H[k], p.Hp[k], s.L[k]);
-      }
-      DTB_LAUNCH_OK();
-    }
     woff += chunk * s.F;
     soff += (size_t)B * s.D * s.L[k];
     if ((int)chunk > bstage) bstage = (int)chunk;
   }
   p.b_stage_bytes = bstage;
-  p.wmax = stats;
+  // statistics words of the single fp16 pass, read by the cin_tc2.cu kernels: [k] max|W_k|, [8 + k] max|dC_k|,
+  // [16] max|x0|, [24 + k] max|h_k| (bit patterns of non-negative floats)
+  int* stats = reinterpret_cast<int*>(ws + bwd_stats_end(s, B) - 256);
   if (f16) {
-    f16_v2 = !g_tc_f16_v1 && cin_tc2_bwd_supported(p, s.D);
-    if (!f16_v2) {
+    // the two-threads-per-row data-gradient kernel of cin_tc2.cu, whose fp16 dC tiles its weight-gradient kernel reads
+    if (!cin_tc2_bwd_supported(p, s.D)) {
       set_error("dtb_cin_bwd: fp16 single pass: shape outside cin_tc2 (F=%d D=%d); use precision 0/2", s.F, s.D);
       return DTB_ERR_UNSUPPORTED;
     }
-    f16w = true;
+    float* dpmax = reinterpret_cast<float*>(ws + bwd_stats_end(s, B));
+    p.wmax = stats;
     p.dpmax = dpmax;
     if (phase != 2) {
       const int rcd = cin_tc2_dpmax(d_pooled, dpmax, s.pcol0, s.pool_n, B, s.P, s.n_layers, st);
@@ -1619,72 +1382,57 @@ int cin_tc_bwd(const CinShape& s, const int32_t* idx, const float* table, const 
         const int64_t n_w = (int64_t)s.F * s.H[k] * s.L[k];
         cin_tc_wmax_kernel<<<(int)((n_w + 255) / 256 < 64 ? (n_w + 255) / 256 : 64), 256, 0, st>>>(weights + s.w_off[k], n_w, stats + k);
         DTB_LAUNCH_OK();
-        const int64_t total = (int64_t)s.F * s.L[k] * p.Hp[k];
-        int blocks = (int)((total + 255) / 256);
-        if (blocks > sm_count() * 8) blocks = sm_count() * 8;
-        cin_tc_pack_t_f16_kernel<<<blocks, 256, 0, st>>>(weights + s.w_off[k], ws + p.wpack_off[k], s.F, s.H[k], p.Hp[k], s.L[k],
-                                                         stats + k);
+        cin_tc_pack_t_f16_kernel<<<pack_grid(s, p.Hp[k], k), 256, 0, st>>>(weights + s.w_off[k], ws + p.wpack_off[k], s.F, s.H[k], p.Hp[k],
+                                                                 s.L[k], stats + k);
         DTB_LAUNCH_OK();
       }
+      // operand maxima recorded by cin_tc2_fwd_kernel at the head of the saved buffer -> statistics words of the wgrad
+      const int* sv = reinterpret_cast<const int*>(saved);
+      DTB_CUDA_OK(cudaMemcpyAsync(stats + 16, sv, sizeof(int), cudaMemcpyDeviceToDevice, st));
+      DTB_CUDA_OK(cudaMemcpyAsync(stats + 24, sv, sizeof(int) * s.n_layers, cudaMemcpyDeviceToDevice, st));
+      const int rc = cin_tc2_launch_dgrad(p, s.D, st);
+      if (rc != DTB_OK) return rc;
     }
-  }
-  if (!f16 && s.D == 16 && exp_build == 7 && d_bias != nullptr) {
-    set_error("dtb_cin_bwd: experiment build 7 (fp16 tiles) has no bias-gradient kernel; use a CIN without bias");
-    return DTB_ERR_UNSUPPORTED;
-  }
-  if (f16_v2 && phase != 2) {
-    // operand maxima recorded by cin_tc2_fwd_kernel at the head of the saved buffer -> statistics words of the wgrad
-    const int* sv = reinterpret_cast<const int*>(saved);
-    DTB_CUDA_OK(cudaMemcpyAsync(stats + 16, sv, sizeof(int), cudaMemcpyDeviceToDevice, st));
-    DTB_CUDA_OK(cudaMemcpyAsync(stats + 24, sv, sizeof(int) * s.n_layers, cudaMemcpyDeviceToDevice, st));
-  } else if (f16w && phase != 2) {
-    // maxima of the operand tiles the forward saved (the wgrad scale G needs them); padded entries are zeros
-    const size_t blocks64 = m_pad_rows(s, B) / 64;
-    const float* sv = reinterpret_cast<const float*>(saved);
-    size_t pos = cin_fp32_saved_bytes(s, B) / sizeof(float);
+  } else if (phase != 2) {
     for (int k = 0; k < s.n_layers; ++k) {
-      const int64_t n = (int64_t)(blocks64 * (size_t)(k == 0 ? s.F : s.H[k]) * kWgPad);
-      int nb = (int)((n + 255) / 256);
-      if (nb > sm_count() * 8) nb = sm_count() * 8;
-      cin_tc_wmax_kernel<<<nb, 256, 0, st>>>(sv + pos, n, stats + 24 + k);
+      cin_tc_pack_t_kernel<<<pack_grid(s, p.Hp[k], k), 256, 0, st>>>(weights + s.w_off[k], ws + p.wpack_off[k], s.F, s.H[k], p.Hp[k], s.L[k]);
       DTB_LAUNCH_OK();
-      if (k == 0) {
-        cin_tc_wmax_kernel<<<nb, 256, 0, st>>>(sv + pos, n, stats + 16);
-        DTB_LAUNCH_OK();
-      }
-      pos += (size_t)n;          // x0 tiles, then h_1, h_2, ... tiles
     }
+    const int smem = tc_bwd_layout(bstage, s.F).total;
+    int rc = DTB_OK;
+    switch (s.D) {
+      case 4: rc = launch_dgrad<4>(p, smem, st); break;
+      case 8: rc = launch_dgrad<8>(p, smem, st); break;
+      case 16: rc = launch_dgrad<16>(p, smem, st); break;
+      case 32: rc = launch_dgrad<32>(p, smem, st); break;
+      default: set_error("dtb_cin_bwd: embedding dim %d unsupported", s.D); return DTB_ERR_UNSUPPORTED;
+    }
+    if (rc != DTB_OK) return rc;
   }
-  const TcBwdSmemLayout lay = tc_bwd_layout(bstage, s.F);
-  int rc = DTB_OK;
-  if (phase != 2 && f16_v2) {
-    rc = cin_tc2_launch_dgrad(p, s.D, st);
-  } else if (phase != 2) switch (s.D) {
-    case 4: rc = launch_dgrad<4>(p, lay.total, st); break;
-    case 8: rc = launch_dgrad<8>(p, lay.total, st); break;
-    case 16: rc = launch_dgrad<16>(p, lay.total, st); break;
-    case 32: rc = launch_dgrad<32>(p, lay.total, st); break;
-    default: set_error("dtb_cin_bwd: embedding dim %d unsupported", s.D); return DTB_ERR_UNSUPPORTED;
-  }
-  if (rc != DTB_OK || phase == 1) return rc;
+  if (phase == 1) return DTB_OK;
   // ---- wgrad, one launch per layer ------------------------------------------------------------
-  const int R = 128 / s.D;
-  const size_t n_super = ((size_t)B + 2 * R - 1) / (2 * R);
-  const size_t m_pad = n_super * 256;
-  const float* x0t = reinterpret_cast<const float*>(saved);
-  size_t toff = (size_t)B * s.D * s.F;
-  const size_t bt_blocks = m_pad / 64;
-  const size_t xb_pos = cin_fp32_saved_bytes(s, B) / sizeof(float);
-  size_t hb_pos = xb_pos + bt_blocks * s.F * kWgPad;
+  const size_t m_pad = m_pad_rows(s, B);
+  const float* xb = reinterpret_cast<const float*>(saved) + xb_pos;
+  const float* hb = xb + bt_blocks * s.F * kWgPad;
   for (int k = 0; k < s.n_layers; ++k) {
+    const float* hk = k == 0 ? xb : hb;       // block-transposed copies written by the forward kernel
+    if (k > 0) hb += bt_blocks * s.H[k] * kWgPad;
+    const uint8_t* dc = p.dc_tiles + dc_off[k];
+    float* d_w = d_weights + s.w_off[k];
+    const int n_stage_total = (int)(m_pad / kWgStageRows);
+    if (f16) {
+      const int rcw = cin_tc2_launch_wgrad(xb, hk, dc, d_w, s.F, s.H[k], p.Hp[k], s.L[k], n_stage_total, stats, k, st);
+      if (rcw != DTB_OK) return rcw;
+      if (d_bias) {
+        const int rcb = cin_tc2_dbias(dc, d_bias + s.b_off[k], s.L[k], (int)(m_pad / 16), st);
+        if (rcb != DTB_OK) return rcb;
+      }
+      continue;
+    }
     CinTcWgradParams w{};
-    w.xb = x0t + xb_pos;
-    w.hb = k == 0 ? w.xb : x0t + hb_pos;      // block-transposed copies written by the forward kernel
-    if (k > 0) hb_pos += bt_blocks * s.H[k] * kWgPad;
-    w.dc_tiles = p.dc_tiles + dc_off[k];
-    w.d_w = d_weights + s.w_off[k];
+    w.xb = xb; w.hb = hk; w.dc_tiles = dc; w.d_w = d_w;
     w.F = s.F; w.H = s.H[k]; w.Hp = p.Hp[k]; w.L = s.L[k]; w.n_pass = n_pass;
-    w.n_stage_total = (int)(m_pad / kWgStageRows);
+    w.n_stage_total = n_stage_total;
     const int ipt = 128 / w.Hp;
     const int n_tiles = (s.F + ipt - 1) / ipt;
     const int n_pairs = (n_tiles + 1) / 2;
@@ -1694,30 +1442,16 @@ int cin_tc_bwd(const CinShape& s, const int32_t* idx, const float* table, const 
     w.stages_per_split = (w.n_stage_total + splits - 1) / splits;
     splits = (w.n_stage_total + w.stages_per_split - 1) / w.stages_per_split;
     const WgSmemLayout wl = wg_layout(w.L, w.Hp, w.F);
-    if (f16_v2) {
-      const int rcw = cin_tc2_launch_wgrad(w.xb, w.hb, w.dc_tiles, w.d_w, w.F, w.H, w.Hp, w.L, w.n_stage_total, stats, k, st);
-      if (rcw != DTB_OK) return rcw;
-    } else if (f16w) {
-      w.stats = stats;
-      w.layer = k;
-      DTB_CUDA_OK(cudaFuncSetAttribute(cin_tc_wgrad_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, wl.total));
-      cin_tc_wgrad_kernel<true><<<dim3(n_pairs, splits), kWgThreads, wl.total, st>>>(w);
-    } else {
-      DTB_CUDA_OK(cudaFuncSetAttribute(cin_tc_wgrad_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, wl.total));
-      cin_tc_wgrad_kernel<false><<<dim3(n_pairs, splits), kWgThreads, wl.total, st>>>(w);
-    }
-    if (!f16_v2) DTB_LAUNCH_OK();
-    if (d_bias && f16w) {
-      const int rcb = cin_tc2_dbias(w.dc_tiles, d_bias + s.b_off[k], w.L, (int)(m_pad / 16), st);
-      if (rcb != DTB_OK) return rcb;
-    } else if (d_bias) {
+    DTB_CUDA_OK(cudaFuncSetAttribute(cin_tc_wgrad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, wl.total));
+    cin_tc_wgrad_kernel<<<dim3(n_pairs, splits), kWgThreads, wl.total, st>>>(w);
+    DTB_LAUNCH_OK();
+    if (d_bias) {
       const int n_blocks16 = (int)(m_pad / 16);
       int blocks = (int)(((int64_t)n_blocks16 * w.L + 255) / 256);
       if (blocks > sm_count() * 8) blocks = sm_count() * 8;
-      cin_tc_dbias_kernel<<<blocks, 256, 0, st>>>(w.dc_tiles, d_bias + s.b_off[k], w.L, n_blocks16);
+      cin_tc_dbias_kernel<<<blocks, 256, 0, st>>>(dc, d_bias + s.b_off[k], w.L, n_blocks16);
       DTB_LAUNCH_OK();
     }
-    toff += (size_t)B * s.D * s.L[k];
   }
   return DTB_OK;
 }

@@ -1,8 +1,9 @@
 // CIN on tcgen05, second organisation: ONE tensor pass on power-of-two-scaled fp16 operands (DTB_CIN_TC_F16X1) with
 // TWO threads per GEMM row.
 //
-// Why a second organisation.  With a single tensor pass the MMA work of cin_tc_fwd_kernel<D, true> drops to a third,
-// but its time only fell from 2.54 to 1.90 ms (B200, 65 536 rows): the kernel was never waiting for the tensor pipe any
+// Why a second organisation.  With a single tensor pass the MMA work of a one-thread-per-row fp16 forward built like
+// cin_tc_fwd_kernel<D> (cin_tc.cu; removed, it remains in git history at commit 021caee) dropped to a third, but its
+// time only fell from 2.54 to 1.90 ms (B200, 65 536 rows): the kernel was never waiting for the tensor pipe any
 // more, it was waiting for ITSELF -- 130 pipeline granules per super tile, each a serial chain
 // (products -> wait empty -> tcgen05.st -> wait::st -> arrive -> MMA issuer: wait tile 0, issue, wait tile 1, issue, 2 commits)
 // of roughly a thousand cycles for 256 cycles of tensor work.  Here:
@@ -16,8 +17,7 @@
 //     two (halves the epilogue, which nothing overlaps because the next layer's operand depends on it);
 //   * the fp16 operand of a granule is 32 TMEM columns per tile: 4 stages x 2 tiles = 256 columns next to the two
 //     128-column accumulators (TMEM 100 % allocated, as before).
-// Arithmetic, saved-activation format and the weight images are exactly those of cin_tc_fwd_kernel<D, true>
-// (cin_tc.cu): per-row scale 2^e chosen from max|x0 row| * max|h row| (the two halves exchange their maxima through
+// Arithmetic: per-row scale 2^e chosen from max|x0 row| * max|h row| (the two halves exchange their maxima through
 // shared memory), per-layer weight scale from max|W_k|, both undone on the fp32 accumulator.
 #include "cin_tc_common.cuh"
 #include <cuda_fp16.h>
@@ -734,13 +734,14 @@ __global__ void cin_tc2_dbias_kernel(const uint8_t* __restrict__ dc_tiles, float
 }
 
 // ==========================================================================================
-// Backward, weight gradient on ONE fp16 pass (the counterpart of cin_tc_wgrad_kernel<true>, cin_tc.cu)
+// Backward, weight gradient on ONE fp16 pass
 // ==========================================================================================
 //   dW_k[(i,j), l] = sum_m x0[m,i] h_k[m,j] dC_k[m,l]     UMMA M = (i,j) pairs, K = batch x dim rows m, N = L
 // The reduction runs over m, so per-row scales must cancel inside the MMA: the dC tile row m carries t_m, the
 // on-the-fly operand A'[(i,j), m] = x0[m,i] h[m,j] (G / t_m) its inverse and ONE per-layer G (from the recorded maxima)
-// keeps |A'| < 1024.  What changed against cin_tc_wgrad_kernel<true> (1.94 ms for the three layers, tensor pipe 32 %,
-// producers issue-bound: 3 multiplies + operand fetches per element in 256 threads):
+// keeps |A'| < 1024.  What changed against a first fp16 version built like cin_tc_wgrad_kernel (removed, in git history
+// at commit 021caee; 1.94 ms for the three layers, tensor pipe 32 %, producers issue-bound: 3 multiplies + operand
+// fetches per element in 256 threads):
 //   * a SCALER warp multiplies the x0 tile of a stage by G / t_m once (F x 64 products) -- the 256 producer threads then
 //     do ONE multiply per element (x' h) instead of three;
 //   * one MMA-issuing warp per tile; 4 operand stages (an fp16 operand block is 32 TMEM columns, not 64);

@@ -31,9 +31,8 @@ struct CinTcParams {
   unsigned long long xb_off;                     // float offset of the block-transposed copy of x0
   unsigned long long bias_off[kCinMaxLayers];
   int b_stage_bytes;                              // bytes reserved per weight stage in smem
-  int dbg;                                        // profiling switches (tools/bench_cin.py): 1 no produce, 2 no MMA, 4 no epilogue
   int compact;                                    // training: save relu-mask bits instead of the fp32 T_k rows (see cin_tc_compact)
-  const int* wmax;                                // fp16 variant only: bit pattern of max|W_k| per layer (cin_tc_wmax_kernel)
+  const int* wmax;                                // cin_tc2: bit pattern of max|W_k| per layer (cin_tc_wmax_kernel)
 };
 
 static inline int round_up(int x, int m) { return (x + m - 1) / m * m; }
@@ -72,7 +71,7 @@ struct CinTcBwdParams {
   unsigned long long hb_off[kCinMaxLayers];      // float offset of the block-transposed h_{k+1} tiles (as in CinTcParams)
   int b_stage_bytes;
   int compact;                                    // saved activations in the compact format (cin_tc_compact)
-  const int* wmax;                                // fp16 variants: statistics words (max|W_k| per layer at [k], max|dC_k| at [8 + k])
+  const int* wmax;                                // cin_tc2: statistics words (max|W_k| per layer at [k], max|dC_k| at [8 + k])
   const float* dpmax;                             // cin_tc2: max|d_pooled[b, pooled columns of layer k]|, [B, n_layers]
 };
 

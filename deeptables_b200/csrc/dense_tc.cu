@@ -16,13 +16,12 @@
 // -> tcgen05.mma (SS form), 4-stage mbarrier ring, weights by bulk async copy, double-buffered TMEM accumulators whose
 // read-out (bias / relu; lane = output row, 32 columns per TMEM read written as 8 float4 of the lane's own 128-byte line)
 // overlaps the next tile's loads.  Outputs whose rows are not 16-byte aligned go through a shared-memory transpose instead
-// (also selectable with DTB_DENSE_DIRECT=0: it was the only form until the [B*F, 32] -> 128 AutoInt projection measured
-// 0.82 ms against 0.44 ms for the direct stores).
+// (it was the only form until the [B*F, 32] -> 128 AutoInt projection measured 0.82 ms against 0.44 ms for the direct
+// stores).
 #include "dtb_common.cuh"
 #include "tcgen05.cuh"
 #include "dense_tc.h"
 #include <cuda_bf16.h>
-#include <cstdlib>
 
 namespace dtb {
 
@@ -555,12 +554,8 @@ int dense_tc_rows(const float* A, int lda, const float* W, int ldw, int transpos
   p.A = A; p.wpack = reinterpret_cast<const uint8_t*>(workspace); p.bias = bias; p.out = out;
   p.M = M; p.K = K; p.Nout = Nout; p.lda = lda; p.ldo = ldo; p.NT = t.NT; p.n_tiles = t.n_tiles; p.n_chunks = t.n_chunks;
   p.act = act;
-  {
-    static const int mode = [] { const char* e = getenv("DTB_DENSE_DIRECT"); return e ? atoi(e) : 1; }();   // 0: transposed
-    const bool ok = Nout % 4 == 0 && ldo % 4 == 0 && (reinterpret_cast<uintptr_t>(out) & 15) == 0 &&
-                    (!bias || (reinterpret_cast<uintptr_t>(bias) & 15) == 0);
-    p.direct = (mode != 0 && ok) ? 1 : 0;
-  }
+  p.direct = (Nout % 4 == 0 && ldo % 4 == 0 && (reinterpret_cast<uintptr_t>(out) & 15) == 0 &&
+              (!bias || (reinterpret_cast<uintptr_t>(bias) & 15) == 0)) ? 1 : 0;
   const DtSmem lay = dt_layout(t.NT, 1);
   DTB_CUDA_OK(cudaFuncSetAttribute(dense_tc_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, lay.total));
   const int n_items = ((M + 127) / 128) * t.n_tiles;

@@ -7,7 +7,6 @@
 // with the filter in shared memory (read as 128-bit warp broadcasts) -- 43 GFLOP per 65 536-row step at the reference's
 // defaults (14 / 16 filters, height 7) against 1.5 GB of activations, i.e. bandwidth and issue bound, not a tensor-core shape.
 #include "dtb_common.cuh"
-#include <cstdlib>
 
 namespace dtb {
 
@@ -124,64 +123,11 @@ __global__ void __launch_bounds__(kFgThreads) conv_fields_bwd_dx_kernel(const fl
   }
 }
 
-#ifdef DTB_FIRST_VERSIONS
-// (first filter-gradient kernel, compiled only with -DDTB_FIRST_VERSIONS)
-// dK[t,ci,co] += sum_pos X[b, h + t - pad, w, ci] dZ[b,h,w,co];  dbias[co] += sum_pos dZ.  A thread owns up to 4 (ci, co)
-// entries with their kh taps in registers and streams the CTA's positions; lanes run over co (dZ reads coalesced, X reads
-// are broadcasts).  One atomic per filter element per CTA.
-__global__ void __launch_bounds__(kFgThreads) conv_fields_bwd_dw_kernel(const float* __restrict__ X, const float* __restrict__ Y,
-                                                                        const float* __restrict__ dY, float* __restrict__ dK,
-                                                                        float* __restrict__ dbias, int64_t n_pos, int H, int W,
-                                                                        int Cin, int Cout, int kh, int act,
-                                                                        int64_t pos_per_cta) {
-  const int n_e = Cin * Cout;
-  const int pad = fg_pad_before(H, kh, 1);
-  int ci[4], co[4];
-  float acc[4][kFgMaxKh], accb[4];
-#pragma unroll
-  for (int s = 0; s < 4; ++s) {
-    const int e = threadIdx.x + s * kFgThreads;
-    ci[s] = e < n_e ? e / Cout : -1;
-    co[s] = e < n_e ? e % Cout : 0;
-    accb[s] = 0.f;
-#pragma unroll
-    for (int t = 0; t < kFgMaxKh; ++t) acc[s][t] = 0.f;
-  }
-  const int64_t p_begin = (int64_t)blockIdx.x * pos_per_cta;
-  const int64_t p_end = p_begin + pos_per_cta < n_pos ? p_begin + pos_per_cta : n_pos;
-  for (int64_t pos = p_begin; pos < p_end; ++pos) {
-    const int w = (int)(pos % W);
-    const int64_t bh = pos / W;
-    const int h = (int)(bh % H);
-#pragma unroll
-    for (int s = 0; s < 4; ++s) {
-      if (ci[s] < 0) continue;
-      const float dz = __ldg(dY + pos * Cout + co[s]) * fg_act_grad(__ldg(Y + pos * Cout + co[s]), act);
-      if (ci[s] == 0) accb[s] += dz;
-#pragma unroll
-      for (int t = 0; t < kFgMaxKh; ++t) {
-        const int hh = h + t - pad;
-        if (t < kh && hh >= 0 && hh < H) acc[s][t] = fmaf(__ldg(X + ((bh - h + hh) * W + w) * Cin + ci[s]), dz, acc[s][t]);
-      }
-    }
-  }
-#pragma unroll
-  for (int s = 0; s < 4; ++s) {
-    if (ci[s] < 0) continue;
-#pragma unroll
-    for (int t = 0; t < kFgMaxKh; ++t)
-      if (t < kh && acc[s][t] != 0.f) atomicAdd(dK + ((size_t)t * Cin + ci[s]) * Cout + co[s], acc[s][t]);
-    if (ci[s] == 0 && dbias && accb[s] != 0.f) atomicAdd(dbias + co[s], accb[s]);
-  }
-}
-
-#endif  // DTB_FIRST_VERSIONS
-
-// The same gradient with the positions in parallel: a CTA takes tiles of kFgTile consecutive positions, stages their taps
-// xs[p][a] (a = t Cin + ci, zero outside the block) and dzs[p][co] in shared memory, and every thread accumulates its
-// (a, co) entries -- dK is exactly the [A x Cout] matrix xs^T dzs in memory order -- over the tile; accumulators live in
-// registers across the CTA's tiles, one atomic per entry per CTA at the end.  (The first version above walks the positions
-// serially with one (ci, co) entry per thread: 106 ms per launch at 65 536 rows, 14 live threads per CTA in layer 1.)
+// dK[t,ci,co] += sum_pos X[b, h + t - pad, w, ci] dZ[b,h,w,co];  dbias[co] += sum_pos dZ.  A CTA takes tiles of kFgTile
+// consecutive positions, stages their taps xs[p][a] (a = t Cin + ci, zero outside the block) and dzs[p][co] in shared
+// memory, and every thread accumulates its (a, co) entries -- dK is exactly the [A x Cout] matrix xs^T dzs in memory order --
+// over the tile; accumulators live in registers across the CTA's tiles, one atomic per entry per CTA at the end.  (A first
+// version that walked the positions serially with one (ci, co) entry per thread took 106 ms per launch at 65 536 rows.)
 constexpr int kFgTile = 128;
 constexpr int kFgMaxEntries = 32;        // (kh Cin Cout) / 256 threads, kh <= 8, Cin, Cout <= 32
 
@@ -365,28 +311,13 @@ int dtb_conv_fields_bwd(const float* X, const float* kernel, const float* Y, con
     })
     DTB_LAUNCH_OK();
   }
-  // DTB_FGCNN_DW=0 selects the first (serial-per-CTA) filter-gradient kernel (builds with -DDTB_FIRST_VERSIONS only)
-  static const int tiled = [] { const char* e = getenv("DTB_FGCNN_DW"); return e ? atoi(e) : 1; }();
-  if (tiled) {
-    const int64_t n_tiles = (n_pos + kFgTile - 1) / kFgTile;
-    const size_t smem = (size_t)kFgTile * (kh * Cin + Cout) * sizeof(float);
-    int64_t ctas = (int64_t)sm_count() * 2;
-    if (ctas > n_tiles) ctas = n_tiles;
-    DTB_CUDA_OK(cudaFuncSetAttribute(conv_fields_bwd_dw_tiled_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    conv_fields_bwd_dw_tiled_kernel<<<(int)ctas, kFgThreads, smem, st>>>(X, Y, dY, d_kernel, d_bias, n_pos, H, W, Cin, Cout, kh, act,
-                                                                         n_tiles);
-  } else {
-#ifdef DTB_FIRST_VERSIONS
-    int64_t ctas = (int64_t)sm_count() * 4;
-    if (ctas > n_pos) ctas = n_pos;
-    const int64_t per = (n_pos + ctas - 1) / ctas;
-    ctas = (n_pos + per - 1) / per;
-    conv_fields_bwd_dw_kernel<<<(int)ctas, kFgThreads, 0, st>>>(X, Y, dY, d_kernel, d_bias, n_pos, H, W, Cin, Cout, kh, act, per);
-#else
-    set_error("dtb_conv_fields_bwd: DTB_FGCNN_DW=0 needs a library built with -DDTB_FIRST_VERSIONS");
-    return DTB_ERR_UNSUPPORTED;
-#endif
-  }
+  const int64_t n_tiles = (n_pos + kFgTile - 1) / kFgTile;
+  const size_t smem = (size_t)kFgTile * (kh * Cin + Cout) * sizeof(float);
+  int64_t ctas = (int64_t)sm_count() * 2;
+  if (ctas > n_tiles) ctas = n_tiles;
+  DTB_CUDA_OK(cudaFuncSetAttribute(conv_fields_bwd_dw_tiled_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  conv_fields_bwd_dw_tiled_kernel<<<(int)ctas, kFgThreads, smem, st>>>(X, Y, dY, d_kernel, d_bias, n_pos, H, W, Cin, Cout, kh, act,
+                                                                       n_tiles);
   DTB_LAUNCH_OK();
   return DTB_OK;
 }

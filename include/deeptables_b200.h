@@ -222,7 +222,7 @@ int dtb_cin_bwd_phase(const int32_t* idx, const float* table, const int64_t* row
  *       fields) -- error ~2e-4 of the output scale, inside the 1e-3 parity bar; shapes outside it fall to 2, then to 1;
  *   1 = the any-shape materialising formulation (outer product in HBM chunks + the bf16x3 GEMMs of csrc/dense_tc.cu);
  *   2 = tensor-core bf16x3 split (hi*hi + lo*hi + hi*lo, ~2^-16 per product: fp32-grade); 3 = one bf16 pass (4e-3: tests only);
- *   4 = force the single fp16 pass (error when the shape is outside it). */
+ *   4 = force the single fp16 pass (DTB_ERR_UNSUPPORTED from forward and backward when the shape is outside it). */
 #define DTB_CIN_AUTO 0
 #define DTB_CIN_FP32 1
 #define DTB_CIN_TC_BF16X3 2
@@ -231,10 +231,12 @@ int dtb_cin_bwd_phase(const int32_t* idx, const float* table, const int64_t* row
 int dtb_cin_tc_supported(int F, int D, const int* layer_sizes_host, int n_layers, int direct);
 /* which of the codes 1 / 2 / 4 a forward + backward with `precision` runs for this shape (0 = auto is resolved) */
 int dtb_cin_resolved_precision(int F, int D, const int* layer_sizes_host, int n_layers, int direct, int precision);
-/* Test hooks for the tensor-core path.  set_variant: 1 (default) feeds the on-the-fly A operand to
- * tcgen05.mma through TMEM, 0 through shared memory.  selftest: C[128,N] = bf16(A[128,K]) @
- * bf16(Bmat[K,N]) with one M=128 UMMA tile (N <= 128, K <= 64, multiples of 16); workspace >= 4*N*K bytes. */
-int dtb_cin_tc_set_variant(int a_operand_in_tmem);
+/* Test hooks for the tensor-core path.  set_variant: process-wide flags read by later CIN calls; bit 0 is
+ * accepted and ignored, bit 16 runs the exact-fp32 backward after a tensor-core forward, bit 17 keeps the full
+ * (fp32 T_k) saved-activation format.  Any other bit returns DTB_ERR_INVALID_ARG and leaves the flags unchanged.
+ * selftest: C[128,N] = bf16(A[128,K]) @ bf16(Bmat[K,N]) with one M=128 UMMA tile (N <= 128, K <= 64, multiples
+ * of 16), the A operand through TMEM (a_operand_in_tmem = 1) or shared memory (0); workspace >= 4*N*K bytes. */
+int dtb_cin_tc_set_variant(int flags);
 int dtb_tc_selftest(const float* A, const float* Bmat, float* C, void* workspace, int N, int K,
                     int a_operand_in_tmem, void* stream);
 

@@ -177,6 +177,15 @@ def test_ctypes_signatures_match_the_header_prototypes():
     assert seen == set(nat._SIGNATURES), sorted(set(nat._SIGNATURES) ^ seen)
 
 
+def test_cin_tc_set_variant_rejects_unknown_bits():
+    """dtb_cin_tc_set_variant knows bits 0, 16 and 17 only: any other bit is an error that names the bit and
+    leaves the flags as they were.  It touches no device."""
+    from deeptables_b200 import _native as nat
+    assert nat.lib.dtb_cin_tc_set_variant(1 | (1 << 12)) == -1          # DTB_ERR_INVALID_ARG
+    assert 'bit 12' in nat.last_error()
+    assert nat.lib.dtb_cin_tc_set_variant(1) == 0
+
+
 def test_no_undefined_globals_in_gpu_only_code():
     """Function bodies of the host modules, bench.py and the GPU tests only execute on a GPU box; catch typos in
     global names here (the image has no pyflakes): tools/lint_names.py."""

@@ -531,44 +531,62 @@ TC_CASES = [  # (F, D, sizes, direct, bias, act, B)
 
 
 @pytest.mark.parametrize('f,d,sizes,direct,use_bias,act,b', TC_CASES)
-@pytest.mark.parametrize('variant', [1, 0])
 @pytest.mark.parametrize('precision', [2, 3])
-def test_cin_tensor_core_forward(nat, f, d, sizes, direct, use_bias, act, b, variant, precision):
+def test_cin_tensor_core_forward(nat, f, d, sizes, direct, use_bias, act, b, precision):
     sizes_c = nat.int_array(sizes)
     n = len(sizes)
-    nat.lib.dtb_cin_tc_set_variant(variant)
-    try:
-        if not nat.lib.dtb_cin_tc_supported(f, d, sizes_c, n, int(direct)):
-            pytest.skip('shape not supported by this tensor-core variant')
-        vocab = [9 + i for i in range(f)]
-        tabs, flat, offs = make_table(vocab, d, seed=21)
-        idx = make_idx(vocab, b, seed=22)
-        g = np.random.default_rng(23)
-        fns = L.cin_field_nums(f, sizes, direct)
-        filt = [(g.normal(size=(f * fns[k], s)) / np.sqrt(f * fns[k])).astype(np.float32) for k, s in enumerate(sizes)]
-        bias = [g.normal(size=s).astype(np.float32) * 0.1 for s in sizes] if use_bias else None
-        wcat = np.concatenate([x.reshape(-1) for x in filt])
-        pw = L.cin_pooled_width(f, dict(cross_layer_size=sizes, direct=direct))
-        pooled = torch.full((b, pw), float('nan'), device='cuda')
-        ws_bytes = nat.lib.dtb_cin_workspace_bytes(b, f, d, sizes_c, n, int(direct), 1)
-        ws = torch.empty(ws_bytes, dtype=torch.uint8, device='cuda')
-        saved = torch.empty(nat.lib.dtb_cin_saved_bytes(b, f, d, sizes_c, n, int(direct)), dtype=torch.uint8, device='cuda')
-        d_b = dev(np.concatenate(bias)) if use_bias else None
-        nat.check(nat.lib.dtb_cin_fwd(P(dev(idx)), P(dev(flat)), P(dev(offs)), P(dev(wcat)), P(d_b), P(pooled), P(saved),
-                                      P(ws), ws_bytes, b, f, d, sizes_c, n, int(direct), act, precision, None, None))
-        torch.cuda.synchronize()
-        x = torch.cat(L.embedding_lookup([torch.tensor(t, dtype=torch.float64) for t in tabs], torch.tensor(idx)), dim=1)
-        want = _cin_oracle(x, sizes, direct, [torch.tensor(w_, dtype=torch.float64) for w_ in filt],
-                           [torch.tensor(b_, dtype=torch.float64) for b_ in bias] if use_bias else None, act).numpy()
-        got = pooled.cpu().numpy()
-        scale = np.abs(want).max()
-        err = np.abs(got - want).max() / scale
-        # bf16x3 split: fp32-grade; single bf16 pass: ~2^-8 per operand
-        assert err < (2e-5 if precision == 2 else 2e-2), f'max err / scale = {err:.3e}'
-        if precision == 2:
-            np.testing.assert_allclose(got, want, rtol=1e-3, atol=1e-4 * scale)
-    finally:
-        nat.lib.dtb_cin_tc_set_variant(1)
+    if not nat.lib.dtb_cin_tc_supported(f, d, sizes_c, n, int(direct)):
+        pytest.skip('shape not supported by the tensor-core kernels')
+    vocab = [9 + i for i in range(f)]
+    tabs, flat, offs = make_table(vocab, d, seed=21)
+    idx = make_idx(vocab, b, seed=22)
+    g = np.random.default_rng(23)
+    fns = L.cin_field_nums(f, sizes, direct)
+    filt = [(g.normal(size=(f * fns[k], s)) / np.sqrt(f * fns[k])).astype(np.float32) for k, s in enumerate(sizes)]
+    bias = [g.normal(size=s).astype(np.float32) * 0.1 for s in sizes] if use_bias else None
+    wcat = np.concatenate([x.reshape(-1) for x in filt])
+    pw = L.cin_pooled_width(f, dict(cross_layer_size=sizes, direct=direct))
+    pooled = torch.full((b, pw), float('nan'), device='cuda')
+    ws_bytes = nat.lib.dtb_cin_workspace_bytes(b, f, d, sizes_c, n, int(direct), 1)
+    ws = torch.empty(ws_bytes, dtype=torch.uint8, device='cuda')
+    saved = torch.empty(nat.lib.dtb_cin_saved_bytes(b, f, d, sizes_c, n, int(direct)), dtype=torch.uint8, device='cuda')
+    d_b = dev(np.concatenate(bias)) if use_bias else None
+    nat.check(nat.lib.dtb_cin_fwd(P(dev(idx)), P(dev(flat)), P(dev(offs)), P(dev(wcat)), P(d_b), P(pooled), P(saved),
+                                  P(ws), ws_bytes, b, f, d, sizes_c, n, int(direct), act, precision, None, None))
+    torch.cuda.synchronize()
+    x = torch.cat(L.embedding_lookup([torch.tensor(t, dtype=torch.float64) for t in tabs], torch.tensor(idx)), dim=1)
+    want = _cin_oracle(x, sizes, direct, [torch.tensor(w_, dtype=torch.float64) for w_ in filt],
+                       [torch.tensor(b_, dtype=torch.float64) for b_ in bias] if use_bias else None, act).numpy()
+    got = pooled.cpu().numpy()
+    scale = np.abs(want).max()
+    err = np.abs(got - want).max() / scale
+    # bf16x3 split: fp32-grade; single bf16 pass: ~2^-8 per operand
+    assert err < (2e-5 if precision == 2 else 2e-2), f'max err / scale = {err:.3e}'
+    if precision == 2:
+        np.testing.assert_allclose(got, want, rtol=1e-3, atol=1e-4 * scale)
+
+
+def test_cin_fp16_forward_outside_cin_tc2_is_unsupported(nat):
+    """Precision 4 forces the single fp16 pass, which only the cin_tc2 kernels run.  On a shape they reject (a
+    hidden half of 8 fields: not a multiple of 16) but the bf16x3 kernels take, the forward returns
+    DTB_ERR_UNSUPPORTED before it launches anything: workspace and output stay untouched."""
+    f, d, sizes, b = 26, 16, (16, 16), 40
+    sizes_c, n = nat.int_array(sizes), len(sizes)
+    assert nat.lib.dtb_cin_tc_supported(f, d, sizes_c, n, 0)
+    vocab = [9 + i for i in range(f)]
+    _, flat, offs = make_table(vocab, d, seed=24)
+    idx = make_idx(vocab, b, seed=25)
+    fns = L.cin_field_nums(f, sizes, False)
+    wcat = np.concatenate([np.ones(f * fns[k] * s, np.float32) for k, s in enumerate(sizes)])
+    pw = L.cin_pooled_width(f, dict(cross_layer_size=sizes, direct=False))
+    pooled = torch.full((b, pw), float('nan'), device='cuda')
+    ws_bytes = nat.lib.dtb_cin_workspace_bytes(b, f, d, sizes_c, n, 0, 0)
+    ws = torch.full((ws_bytes,), 0x5a, dtype=torch.uint8, device='cuda')
+    rc = nat.lib.dtb_cin_fwd(P(dev(idx)), P(dev(flat)), P(dev(offs)), P(dev(wcat)), None, P(pooled), None, P(ws), ws_bytes,
+                             b, f, d, sizes_c, n, 0, 1, 4, None, None)
+    torch.cuda.synchronize()
+    assert rc == -2 and 'cin_tc2' in nat.last_error()                    # DTB_ERR_UNSUPPORTED
+    assert bool((ws == 0x5a).all()) and bool(pooled.isnan().all())
 
 
 def test_cin_tensor_core_full_batch_properties(nat):

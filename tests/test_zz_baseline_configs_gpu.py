@@ -85,22 +85,18 @@ def test_baseline_config_full_shape(case):
 # ---------------------------------------------------------------------------------------------------------------
 # DTB_CIN_TC_F16X1 (precision code 4): single tensor pass on power-of-two-scaled fp16 operands
 # ---------------------------------------------------------------------------------------------------------------
-F16_CASES = [  # (F, sizes, direct, bias, act, B, D, kernel): 'v2' = two threads per GEMM row (cin_tc2.cu), 'v1' = cin_tc.cu (D = 16)
-    (26, (128, 128, 128), False, False, 1, 37, 16, 'v2'),
-    (26, (128, 128, 128), False, False, 1, 37, 16, 'v1'),
-    (26, (32, 32, 16), False, True, 1, 64, 16, 'v2'),
-    (26, (32, 32, 16), False, True, 1, 64, 16, 'v1'),
-    (10, (64, 32), True, True, 1, 50, 16, 'v2'),
-    (10, (64, 32), True, True, 1, 50, 16, 'v1'),
-    (3, (32, 16), False, False, 0, 9, 16, 'v2'),
-    (3, (32, 16), False, False, 0, 9, 16, 'v1'),
-    (26, (128, 128), False, False, 1, 21, 32, 'v2'),
-    (40, (96, 64, 48), False, True, 1, 300, 16, 'v2'),      # F > 32: layer 0 is a 64-wide chunk too; ragged pooled split
+F16_CASES = [  # (F, sizes, direct, bias, act, B, D): the two-threads-per-GEMM-row kernels of cin_tc2.cu
+    (26, (128, 128, 128), False, False, 1, 37, 16),
+    (26, (32, 32, 16), False, True, 1, 64, 16),
+    (10, (64, 32), True, True, 1, 50, 16),
+    (3, (32, 16), False, False, 0, 9, 16),
+    (26, (128, 128), False, False, 1, 21, 32),
+    (40, (96, 64, 48), False, True, 1, 300, 16),      # F > 32: layer 0 is a 64-wide chunk too; ragged pooled split
 ]
 
 
-@pytest.mark.parametrize('f,sizes,direct,use_bias,act,b,d,kernel', F16_CASES)
-def test_cin_fp16_single_pass_forward_is_inside_the_parity_bar(f, sizes, direct, use_bias, act, b, d, kernel):
+@pytest.mark.parametrize('f,sizes,direct,use_bias,act,b,d', F16_CASES)
+def test_cin_fp16_single_pass_forward_is_inside_the_parity_bar(f, sizes, direct, use_bias, act, b, d):
     """tools/cin_precision_study.py predicts max |err| of 2-6e-4 of the output scale for this scheme; the parity
     bar is rtol 1e-3 (+ atol 1e-4 of the scale).  Also checks that a backward (bf16x3 kernels) runs on the
     activations this forward saved."""
@@ -129,13 +125,9 @@ def test_cin_fp16_single_pass_forward_is_inside_the_parity_bar(f, sizes, direct,
     ws_bytes = nat.lib.dtb_cin_workspace_bytes(b, f, d, sizes_c, n, int(direct), 1)
     ws = torch.empty(ws_bytes, dtype=torch.uint8, device='cuda')
     saved = torch.empty(nat.lib.dtb_cin_saved_bytes(b, f, d, sizes_c, n, int(direct)), dtype=torch.uint8, device='cuda')
-    nat.lib.dtb_cin_tc_set_variant(1 | ((1 << 18) if kernel == 'v1' else 0))
-    try:
-        nat.check(nat.lib.dtb_cin_fwd(P(d_idx), P(d_tab), P(d_offs), P(d_w), P(d_b), P(pooled), P(saved), P(ws), ws_bytes,
-                                      b, f, d, sizes_c, n, int(direct), act, 4, None, None), 'cin_fwd fp16x1')
-        torch.cuda.synchronize()
-    finally:
-        nat.lib.dtb_cin_tc_set_variant(1)
+    nat.check(nat.lib.dtb_cin_fwd(P(d_idx), P(d_tab), P(d_offs), P(d_w), P(d_b), P(pooled), P(saved), P(ws), ws_bytes,
+                                  b, f, d, sizes_c, n, int(direct), act, 4, None, None), 'cin_fwd fp16x1')
+    torch.cuda.synchronize()
     # float64 reference of the pooled feature maps (the oracle's CIN up to the sum over D: identity output kernels)
     t64 = torch.tensor(table, dtype=torch.float64)
     x = torch.stack([t64[offs[i] + torch.tensor(idx[:, i].astype(np.int64))] for i in range(f)], dim=1)
@@ -158,7 +150,7 @@ def test_cin_fp16_single_pass_forward_is_inside_the_parity_bar(f, sizes, direct,
     err = np.abs(got - want)
     assert err.max() / scale < 1e-3, f'max error {err.max() / scale:.2e} of the output scale'
     big = np.abs(want) > 1e-2 * scale
-    print(f'fp16x1 {kernel} F={f} sizes={sizes}: max err / scale {err.max() / scale:.2e}, '
+    print(f'fp16x1 F={f} sizes={sizes}: max err / scale {err.max() / scale:.2e}, '
           f'max rel err on entries > 1% of scale {(err[big] / np.abs(want[big])).max():.2e}')
     # elementwise: 1e-3 relative plus 1e-4 of the scale -- except for tiny reductions (F*H < 64 terms per output) where
     # the rounding errors of the few terms do not average out and the norm-wise bound above is all one fp16 pass gives
@@ -169,29 +161,23 @@ def test_cin_fp16_single_pass_forward_is_inside_the_parity_bar(f, sizes, direct,
     # activations (the fp16 forward's: a different forward flips relu-mask bits of near-zero outputs, which moves single
     # gradient rows by percents and says nothing about the backward arithmetic)
     d_dp = torch.randn(b, pw, device='cuda', generator=torch.Generator(device='cuda').manual_seed(5))
-    flags = (1 << 18) if kernel == 'v1' else 0
 
     def backward(prec_b):
-        nat.lib.dtb_cin_tc_set_variant(1 | flags)
-        try:
-            gt = torch.zeros(table.shape, device='cuda')
-            dw = torch.zeros_like(d_w)
-            db = torch.zeros(sum(sizes), device='cuda') if use_bias else None
-            nat.check(nat.lib.dtb_cin_bwd(P(d_idx), P(d_tab), P(d_offs), P(d_w), P(d_dp), P(saved), P(gt), P(dw), P(db), P(ws),
-                                          ws_bytes, b, f, d, sizes_c, n, int(direct), act, prec_b, None), 'cin_bwd')
-            torch.cuda.synchronize()
-            return gt, dw, db
-        finally:
-            nat.lib.dtb_cin_tc_set_variant(1)
+        gt = torch.zeros(table.shape, device='cuda')
+        dw = torch.zeros_like(d_w)
+        db = torch.zeros(sum(sizes), device='cuda') if use_bias else None
+        nat.check(nat.lib.dtb_cin_bwd(P(d_idx), P(d_tab), P(d_offs), P(d_w), P(d_dp), P(saved), P(gt), P(dw), P(db), P(ws),
+                                      ws_bytes, b, f, d, sizes_c, n, int(direct), act, prec_b, None), 'cin_bwd')
+        torch.cuda.synchronize()
+        return gt, dw, db
 
     ref = backward(2)           # bf16x3 explicitly: 0 = auto resolves to the fp16 kernels where they apply
     assert all(bool(torch.isfinite(t_).all()) for t_ in ref if t_ is not None) and float(ref[1].abs().max()) > 0
-    if kernel == 'v2':
-        got_g = backward(4)
-        for name, r_, g_ in zip(('embedding', 'filter', 'bias'), ref, got_g):
-            if r_ is None:
-                continue
-            assert bool(torch.isfinite(g_).all())
-            rel = float((r_ - g_).abs().max() / r_.abs().max())
-            print(f'fp16x1 backward, {name} gradient vs bf16x3 on the same activations: max err / max {rel:.2e}')
-            assert rel < 2e-3, f'{name} gradient off by {rel:.2e} of its maximum'
+    got_g = backward(4)
+    for name, r_, g_ in zip(('embedding', 'filter', 'bias'), ref, got_g):
+        if r_ is None:
+            continue
+        assert bool(torch.isfinite(g_).all())
+        rel = float((r_ - g_).abs().max() / r_.abs().max())
+        print(f'fp16x1 backward, {name} gradient vs bf16x3 on the same activations: max err / max {rel:.2e}')
+        assert rel < 2e-3, f'{name} gradient off by {rel:.2e} of its maximum'

@@ -1,4 +1,4 @@
-"""Time the CIN forward kernel variants at the BASELINE shape (B=65536, 26x16, CIN 128x128x128)."""
+"""Time the bf16x3 and bf16x1 CIN forward at the BASELINE shape (B=65536, 26x16, CIN 128x128x128)."""
 import ctypes
 import os
 import sys
@@ -31,21 +31,18 @@ def run(precision, train):
 
 
 only = os.environ.get('ONLY')
-dbgs = [int(x) for x in os.environ.get('DBG', '0').split(',')]
-for variant, dbg in [(v, d) for v in (1, 0) for d in dbgs]:
-    nat.lib.dtb_cin_tc_set_variant(variant | (dbg << 8))
-    for precision in (2, 3):
-        for train in (0,):
-            tag = f'dbg={dbg} variant={"TMEM" if variant else "SMEM"} pass={"bf16x3" if precision == 2 else "bf16x1"} train={train}'
-            if only and only != f'{variant}{precision}{train}':
-                continue
-            for _ in range(2):
-                run(precision, train)
-            torch.cuda.synchronize()
-            ts = []
-            for _ in range(5):
-                e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-                e0.record(); run(precision, train); e1.record(); torch.cuda.synchronize()
-                ts.append(e0.elapsed_time(e1))
-            t = sorted(ts)[2]
-            print(f'{tag}: {t:.3f} ms  algorithmic {flop / t / 1e9:.0f} TFLOP/s', flush=True)
+for precision in (2, 3):
+    for train in (0,):
+        tag = f'pass={"bf16x3" if precision == 2 else "bf16x1"} train={train}'
+        if only and only != f'{precision}{train}':
+            continue
+        for _ in range(2):
+            run(precision, train)
+        torch.cuda.synchronize()
+        ts = []
+        for _ in range(5):
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            e0.record(); run(precision, train); e1.record(); torch.cuda.synchronize()
+            ts.append(e0.elapsed_time(e1))
+        t = sorted(ts)[2]
+        print(f'{tag}: {t:.3f} ms  algorithmic {flop / t / 1e9:.0f} TFLOP/s', flush=True)

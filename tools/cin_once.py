@@ -1,10 +1,7 @@
 """One training-mode CIN forward + backward at the BASELINE shape: the target of `ncu --set full` captures
 (5 kernels of interest: cin_tc_fwd, cin_tc_dgrad, 3 x cin_tc_wgrad).  FULL=1 selects the full saved-activation
-format (bit 17 of dtb_cin_tc_set_variant) for A/B against the default compact one; DGRAD_EXP=n (1..4) selects an
-experiment build of the data-gradient kernel (see cin_tc_dgrad_kernel: 1 skeleton, 2 read-out only, 3 pipelined
-read-out, 4 no MMA -- their gradients are meaningless, only the time is of interest; 5 keeps dC_hi in shared memory
-6 runs the data-gradient kernel on ONE fp16 pass with per-row scaling, 7 does that for the weight-gradient
-kernels too (fp16 dC tiles): all three are real variants, CHECK=1 compares their gradients with the product kernels')."""
+format (bit 17 of dtb_cin_tc_set_variant) for A/B against the default compact one; PREC sets the CIN precision code;
+CHECKF=1 / CHECKB=1 compare the forward / backward of that precision with the bf16x3 kernels."""
 import ctypes
 import os
 import sys
@@ -32,10 +29,8 @@ d_pooled = torch.randn(B, 256, device='cuda', generator=g) * 1e-3
 ws_bytes = nat.lib.dtb_cin_workspace_bytes(B, F, D, sizes_c, 3, 0, 1)
 ws = torch.empty(ws_bytes, dtype=torch.uint8, device='cuda')
 saved = torch.empty(nat.lib.dtb_cin_saved_bytes(B, F, D, sizes_c, 3, 0), dtype=torch.uint8, device='cuda')
-exp = int(os.environ.get('DGRAD_EXP', 0))
 prec = int(os.environ.get('PREC', 0))          # CIN precision code (4 = fp16 single pass)
-v1 = (1 << 18) if os.environ.get('V1') else 0   # fp16: one-thread-per-row kernels instead of cin_tc2.cu
-nat.lib.dtb_cin_tc_set_variant(1 | ((1 << 17) if os.environ.get('FULL') else 0) | (exp << 12) | v1)
+nat.check(nat.lib.dtb_cin_tc_set_variant(1 | ((1 << 17) if os.environ.get('FULL') else 0)), 'cin_tc_set_variant')
 reps = int(os.environ.get('REPS', 1))
 for rep in range(reps):
     e = [torch.cuda.Event(enable_timing=True) for _ in range(4)]
@@ -50,7 +45,7 @@ for rep in range(reps):
     torch.cuda.synchronize()
     print(f'rep {rep}: fwd {e[0].elapsed_time(e[1]):.3f} ms  dgrad {e[1].elapsed_time(e[2]):.3f} ms  wgrad '
           f'{e[2].elapsed_time(e[3]):.3f} ms  ({"full" if os.environ.get("FULL") else "compact"} saved activations, '
-          f'dgrad experiment {exp}, precision {prec}{" v1" if v1 else ""})', flush=True)
+          f'precision {prec})', flush=True)
 nat.lib.dtb_cin_tc_set_variant(1)
 if os.environ.get('CHECKF'):
     # forward of this precision / kernel against the bf16x3 forward
@@ -75,19 +70,3 @@ if os.environ.get('CHECKB') and prec:
     eg = float((res[0][0] - res[1][0]).abs().max() / res[0][0].abs().max())
     ew = float((res[0][1] - res[1][1]).abs().max() / res[0][1].abs().max())
     print(f'backward precision {prec} vs bf16x3: embedding grad rel err {eg:.2e}, filter grad rel err {ew:.2e}', flush=True)
-if os.environ.get('CHECK') and exp:
-    # gradients of the experiment build against the product kernel on the same saved activations
-    res = []
-    for e_ in (0, exp):
-        nat.lib.dtb_cin_tc_set_variant(1 | ((1 << 17) if os.environ.get('FULL') else 0) | (e_ << 12))
-        grad.zero_()
-        dw.zero_()
-        for phase in (1, 2):
-            nat.check(nat.lib.dtb_cin_bwd_phase(P(idx), P(table), P(offs), P(w), P(d_pooled), P(saved), P(grad), P(dw), None,
-                                                P(ws), ws_bytes, B, F, D, sizes_c, 3, 0, 1, 0, phase, None), 'cin_bwd_phase')
-        torch.cuda.synchronize()
-        res.append((grad.clone(), dw.clone()))
-    nat.lib.dtb_cin_tc_set_variant(1)
-    eg = float((res[0][0] - res[1][0]).abs().max() / res[0][0].abs().max())
-    ew = float((res[0][1] - res[1][1]).abs().max() / res[0][1].abs().max())
-    print(f'experiment {exp} vs product: embedding grad rel err {eg:.2e}, filter grad rel err {ew:.2e}', flush=True)

@@ -1,5 +1,5 @@
 """Time the Dense forward / backward C-ABI calls on the shapes of the bench configs (CUDA events, warm, inputs > L2).
-python tools/dense_once.py  ->  one line per shape; DTB_DENSE_DIRECT=1 selects the lane-per-row epilogue."""
+python tools/dense_once.py  ->  one line per shape."""
 import os
 import sys
 
@@ -43,8 +43,8 @@ def main():
                                                 None), 'b')
         tf, tb = timeit(f), timeit(g)
         gb_f = rows * (i + o) * 4 / 1e9
-        print(f'rows {rows:8d} {i:5d} -> {o:4d}: fwd {tf:7.3f} ms ({gb_f / tf * 1e3:6.0f} GB/s algorithmic)   bwd {tb:7.3f} ms  '
-              f'(direct={os.environ.get("DTB_DENSE_DIRECT", "0")})', flush=True)
+        print(f'rows {rows:8d} {i:5d} -> {o:4d}: fwd {tf:7.3f} ms ({gb_f / tf * 1e3:6.0f} GB/s algorithmic)   bwd {tb:7.3f} ms',
+              flush=True)
         del x, y, dy, dx
 
 

@@ -3,8 +3,7 @@
     python tools/sass_diff.py old.o new.o
 
 Prints which kernels are instruction-identical, which differ and which exist on one side only.  Used to prove that
-adding compile-time experiment variants of a kernel (e.g. cin_tc_dgrad_kernel<16, kExp>) leaves the product
-instantiations byte-for-byte unchanged, so they need no re-validation on the GPU."""
+a source change leaves kernels byte-for-byte unchanged, so they need no re-validation on the GPU."""
 import collections
 import re
 import subprocess
